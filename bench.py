@@ -28,6 +28,8 @@ Prints ONE JSON line on rank 0:
                    its own roofline -- so the driver's records hold them at every N
 `--impl reference` times the CPU implementation alone (rank 0 only under torchrun).
 `--workload c2|c4|c5` makes another BASELINE config the primary line (for profiles/).
+`--dump-outputs DIR` writes the last timed step's answer (see `dump_outputs`) so that two builds
+can be compared output for output: the inputs are seeded, identical from run to run.
 """
 import argparse
 import json
@@ -37,6 +39,7 @@ import sys
 import threading
 import time
 
+sys.dont_write_bytecode = True     # the benchmark writes nothing into the tree it runs from
 os.environ.setdefault("OMP_WAIT_POLICY", "passive")   # see oracle/flatip_oracle.py::_load
 os.environ.setdefault("GOMP_SPINCOUNT", "0")
 
@@ -49,6 +52,7 @@ for p in (ROOT, PKG):
 UNIT = "queries/s"
 CHUNK = 1 << 18          # rows per generated corpus chunk (seeded by global chunk index)
 PROBE_QUERIES = 32       # parity_probe: queries checked against an fp64 brute force per run
+DUMP_BYTES = 60 << 20    # --dump-outputs payload: under 64 MB with the .npy headers
 
 # BASELINE.json configs (SURVEY.md 8d).  bound = the roofline that applies to the scoring kernel.
 WORKLOADS = {
@@ -62,8 +66,10 @@ WORKLOADS = {
 def parse(argv=None):
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=3)
+    ap.add_argument("--steps", type=int, default=None, help="timed steps (default 3; 200 for --workload c5)")
     ap.add_argument("--warmup", type=int, default=3)
+    ap.add_argument("--dump-outputs", default=None, metavar="DIR",
+                    help="write the last timed step's scores / ids as DIR/*.npy (see dump_outputs)")
     ap.add_argument("--impl", default="b2ip", choices=["b2ip", "reference"])
     ap.add_argument("--workload", default="c3", choices=sorted(WORKLOADS))
     ap.add_argument("--n-corpus", type=int, default=None)
@@ -95,8 +101,11 @@ def parse(argv=None):
         if getattr(args, key) is None:
             setattr(args, key, w[key])
     args.bound = w["bound"]
-    if args.workload == "c5" and "--steps" not in (argv if argv is not None else sys.argv):
-        args.steps = 200      # SURVEY 8d: latency per batch over >= 200 batches after warm-up
+    if args.steps is None:
+        # SURVEY 8d: latency per batch over >= 200 batches after warm-up
+        args.steps = 200 if args.workload == "c5" else 3
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be >= 1 and --warmup >= 0")
     return args
 
 
@@ -609,6 +618,35 @@ def run_guarded(fn, torch, dist, world, group):
     return err
 
 
+def dump_rows(np, nq, k):
+    """Query rows whose answers --dump-outputs writes: all of them when their float32 scores and
+    float64 ids fit DUMP_BYTES, else a fixed seeded sample (ascending), the same in every run."""
+    m = min(nq, DUMP_BYTES // (12 * k + 8))
+    if m == nq:
+        return np.arange(nq)
+    return np.sort(np.random.default_rng(0).choice(nq, m, replace=False))
+
+
+def dump_outputs(out_dir, np, D_own, I_own, q_lo, nq, dist=None, group=None):
+    """Writes the answer of a search of `nq` queries -- this rank holds rows [q_lo, q_lo + len(D_own))
+    of it -- for the `dump_rows` queries as out_dir/query_rows.npy (float64 [m]), scores.npy
+    (float32 [m,k]) and ids.npy (float64 [m,k]; exact below 2^53).  With `dist` every rank of
+    `group` must call it; rank 0 gathers the slices and writes."""
+    rows = dump_rows(np, nq, D_own.shape[1])
+    mine = rows[(rows >= q_lo) & (rows < q_lo + D_own.shape[0])]
+    part = (mine.astype(np.float64), np.asarray(D_own[mine - q_lo], dtype=np.float32),
+            np.asarray(I_own[mine - q_lo], dtype=np.float64))
+    if dist is not None:
+        parts = [None] * dist.get_world_size(group) if dist.get_rank() == 0 else None
+        dist.gather_object(part, parts, dst=0, group=group)
+        if dist.get_rank() != 0:
+            return
+        part = tuple(np.concatenate(a) for a in zip(*parts))     # owned slices ascend with the rank
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in zip(("query_rows", "scores", "ids"), part):
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 def main():
     t_start = time.perf_counter()
     args = parse()
@@ -706,6 +744,9 @@ def main():
         torch, D, index, q_dev, k, args.steps, args.warmup, world, sample_clocks_on=local_rank,
         light=(args.bound == "hbm"))
     D_last, I_last, (own_lo, own_hi) = last
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, np, D_last.cpu().numpy(), I_last.cpu().numpy(), own_lo, nq,
+                     *((dist, cpu_group) if world > 1 else ()))
     value = nq / (ms_per_step / 1e3)
     roofline = roofline_of(args, D, agg, args.steps, ms_per_step, hi - lo, nq, args.bound, d)
     def _probe_rows(a, b, ix):

@@ -388,6 +388,71 @@ def test_bench_reference_arm_prints_contract_line():
     assert out.returncode == 0 and out.stdout.strip() == ""
 
 
+def test_bench_steps_sets_the_timed_steps():
+    """--steps is the number of timed steps however it is spelled; only its default depends on the
+    workload (C5: >= 200 batches)."""
+    import bench
+    assert bench.parse([]).steps == 3 and bench.parse(["--workload", "c5"]).steps == 200
+    for argv in (["--steps", "7"], ["--steps=7"], ["--workload", "c5", "--steps=7"], ["--workload=c5", "--steps", "7"]):
+        assert bench.parse(argv).steps == 7, argv
+    for argv in (["--steps", "0"], ["--warmup", "-1"]):
+        with pytest.raises(SystemExit):
+            bench.parse(argv)
+
+
+_DUMP_WORKER = r'''
+import os, sys
+import numpy as np, torch.distributed as dist
+sys.path[:0] = [ROOT]
+import bench
+rank, world = int(os.environ["RANK"]), int(os.environ["WORLD_SIZE"])
+dist.init_process_group("gloo", init_method="tcp://127.0.0.1:" + os.environ["MASTER_PORT"], rank=rank, world_size=world)
+rng = np.random.default_rng(1)
+D = rng.standard_normal((NQ, K)).astype(np.float32)
+I = rng.integers(0, 1 << 40, size=(NQ, K))
+per = -(-NQ // world)
+lo, hi = rank * per, min((rank + 1) * per, NQ)
+bench.dump_outputs(OUT, np, D[lo:hi], I[lo:hi], lo, NQ, dist, None)
+dist.destroy_process_group()
+print("rank", rank, "ok")
+'''
+
+
+@pytest.mark.parametrize("nq,k", [(300, 10), (7000, 1000)])
+def test_bench_dump_outputs_writes_the_sampled_answer(tmp_path, nq, k):
+    """bench.dump_outputs: float32 scores and float64 ids (exact beyond 2^32) of every query when
+    they fit, else of a fixed seeded sample under 64 MB; the same files from one process holding
+    the whole answer and from two ranks each holding a slice (gathered over gloo)."""
+    import bench
+    rng = np.random.default_rng(1)
+    D = rng.standard_normal((nq, k)).astype(np.float32)
+    I = rng.integers(0, 1 << 40, size=(nq, k))
+    rows = bench.dump_rows(np, nq, k)
+    assert np.array_equal(rows, bench.dump_rows(np, nq, k)) and (np.diff(rows) > 0).all()
+    assert (len(rows) == nq) == (nq * k * 12 <= bench.DUMP_BYTES)
+    one = tmp_path / "one"
+    bench.dump_outputs(str(one), np, D, I, 0, nq)
+    got = {n: np.load(one / f"{n}.npy") for n in ("query_rows", "scores", "ids")}
+    assert got["scores"].dtype == np.float32 and got["ids"].dtype == got["query_rows"].dtype == np.float64
+    assert np.array_equal(got["query_rows"], rows) and np.array_equal(got["scores"], D[rows])
+    assert np.array_equal(got["ids"].astype(np.int64), I[rows])
+    assert sum(os.path.getsize(one / f"{n}.npy") for n in got) < 64_000_000
+    script = tmp_path / "dump_worker.py"
+    two = tmp_path / "two"
+    script.write_text(f"ROOT = {ROOT!r}\nOUT = {str(two)!r}\nNQ, K = {nq}, {k}\n" + _DUMP_WORKER)
+    port = str(33000 + os.getpid() % 2000)
+    procs = []
+    for r in range(2):
+        env = dict(os.environ, RANK=str(r), WORLD_SIZE="2", MASTER_ADDR="127.0.0.1", MASTER_PORT=port)
+        procs.append(subprocess.Popen([sys.executable, str(script)], env=env, stdout=subprocess.PIPE,
+                                      stderr=subprocess.STDOUT, text=True))
+    outs = [p.communicate(timeout=300)[0] for p in procs]
+    for r, (p, o) in enumerate(zip(procs, outs)):
+        assert p.returncode == 0 and f"rank {r} ok" in o, o[-3000:]
+    for n in got:
+        assert (two / f"{n}.npy").read_bytes() == (one / f"{n}.npy").read_bytes(), n
+
+
 class _RecordingIndex:
     """Stands in for Indexer: records the index_data call sequence."""
     def __init__(self):
@@ -499,20 +564,6 @@ def test_dropin_launcher_can_swap_a_function_the_script_defines(tmp_path, built)
     out = subprocess.run([sys.executable, "-m", "b2ip.dropin", str(probe)], capture_output=True, text=True,
                          env=env, cwd=str(tmp_path), timeout=120)
     assert out.stdout.split() == ["__main__", "embed_queries"]
-
-
-@pytest.mark.skipif(not os.path.exists("/root/reference/passage_retrieval.py"),
-                    reason="reference checkout not present (GPU box)")
-def test_dropin_launcher_runs_the_unmodified_reference_driver(built):
-    """The real passage_retrieval.py imports and parses its flags under the launcher although
-    faiss is not installed (its `import src.index` resolves to the drop-in)."""
-    import subprocess
-    import sys
-    env = dict(os.environ, PYTHONPATH=os.path.join(ROOT, "czech-contriever_b200"))
-    out = subprocess.run([sys.executable, "-m", "b2ip.dropin", "/root/reference/passage_retrieval.py", "--help"],
-                         capture_output=True, text=True, env=env, cwd="/tmp", timeout=600)
-    assert out.returncode == 0, (out.stdout + out.stderr)[-3000:]
-    assert "--passages_embeddings" in out.stdout and "--n_docs" in out.stdout
 
 
 def test_segment_map_local_to_global(built):
