@@ -28,7 +28,6 @@
 #include "../../include/b2ip.h"
 #include "coarse_kernel.cuh"
 #include "select_kernels.cuh"
-#include "stream_search.cuh"
 
 using namespace b2ip;
 
@@ -101,7 +100,7 @@ struct b2ip_index_s {
     PFN_encodeTiled encode = nullptr;
     // grow-only workspace
     DevBuf q16, eps2, thr, cnt, kept, flags, cand, qstage, qhalf, out_s, out_r, exact_scores, exact_misc,
-        qlist, stage, seg_tab, stream_sync, gmax;
+        qlist, stage, seg_tab, gmax;
     int n_seg = 0;                        // row segments (b2ip_set_row_segments); 0 = row_offset
     std::vector<cudaEvent_t> ev_pool, ev_fin;
     cudaEvent_t ev_t0 = nullptr, ev_t1 = nullptr;
@@ -114,12 +113,6 @@ struct b2ip_index_s {
     int pair = 1;                         // CTA-pair (cta_group::2) scoring kernel when nq > 128
     int stream_kernel = 1;                // nq <= 64: streaming kernel (corpus on the MMA's M side)
     int list_fill_pct = 70;               // adaptive slab schedule: expected list fill after the next slab (% of cap)
-    int stream_coop = 1;                  // cooperative launch of that kernel (co-residency guaranteed)
-    int stream_stages = 8;                // cap on the corpus stages in flight per SM (tuning)
-    int stream_fused = 0;                 // ... with the whole slab schedule + threshold refreshes in ONE launch
-                                          // (stream_search.cuh).  OFF by default: measured, it saves the launch
-                                          // structure (-35 us per batch) but streams 3-4 % slower -- see DESIGN 4.1d
-    long long stream_timeout_ns = 2ll * 1000000000ll;   // bound on every in-kernel wait of that launch
     int bootstrap = 1;                    // nq <= 64: threshold from ONE group-max launch over a corpus sample, then
                                           // one filtered slab over all rows (instead of the geometric slab schedule)
     int bootstrap_max_mb = 64;            // ... while the sample (read twice) is at most this many MiB of 16-bit rows
@@ -689,32 +682,6 @@ void plan_bootstrap(int64_t n, int k, int cap, int sm_count, int d_pad, int max_
     *tiles = boot_tiles;
 }
 
-// Slab sizes of the FIXED geometric schedule of the latency regime (<= 2048 queries): the sequence
-// the launch loop of tensor_search walks through, computed up front for the one-launch streaming
-// search (stream_search.cuh).  `slab` = size of the first slab.
-void plan_fixed_slabs(int64_t n, int64_t slab, int cap, int k, std::vector<int64_t>* out) {
-    out->clear();
-    double growth = 0.0;
-    if (n > slab) {
-        const double r_max = std::max(2.0, 0.5 * cap / (3.0 * k));
-        const double span = static_cast<double>(n) / static_cast<double>(slab);
-        const int steps = std::max(1, static_cast<int>(std::ceil(std::log(span) / std::log(r_max))));
-        growth = std::pow(span, 1.0 / steps);
-    }
-    int64_t done = 0;
-    while (done < n) {
-        int64_t s = std::min<int64_t>(slab, n - done);
-        if (done + s < n) s = std::max<int64_t>(TILE_X, s / TILE_X * TILE_X);
-        s = std::min<int64_t>(s, n - done);
-        out->push_back(s);
-        done += s;
-        if (done >= n) break;
-        if (out->size() > 64) { out->clear(); return; }
-        slab = std::max<int64_t>(TILE_X, static_cast<int64_t>(static_cast<double>(done) * (growth - 1.0)));
-        if (n - done - slab < slab / 4) slab = n - done;          // no tiny tail slab
-    }
-}
-
 int tensor_search(b2ip_handle h, const float* q32, int64_t nq, int k, float* d_scores,
                   int64_t* d_rows) {
     const int64_t n = h->n;
@@ -841,32 +808,11 @@ int tensor_search(b2ip_handle h, const float* q32, int64_t nq, int k, float* d_s
         // padded batch fits next to at least 4 corpus stages in shared memory
         const int nq_s = nqb <= 32 ? 32 : 64;
         const size_t q_bytes = static_cast<size_t>(h->d_pad / KBLOCK_ELEMS) * nq_s * KBLOCK_BYTES;
-        const int stream_stages = static_cast<int>(std::min<long long>(
-            std::min(STREAM_MAX_STAGES, h->stream_stages),
-            (static_cast<long long>(MAX_SMEM_OPTIN) - STREAM_MISC_BYTES - static_cast<long long>(q_bytes)) / STREAM_X_STAGE_BYTES));
-        const bool use_stream = h->stream_kernel && nqb <= 64 && stream_stages >= 4;
-        const size_t stream_smem = static_cast<size_t>(std::max(stream_stages, 0)) * STREAM_X_STAGE_BYTES + q_bytes + STREAM_MISC_BYTES;
+        const int stages = static_cast<int>(std::min<long long>(
+            STREAM_STAGES, (static_cast<long long>(MAX_SMEM_OPTIN) - STREAM_MISC_BYTES - static_cast<long long>(q_bytes)) / STREAM_X_STAGE_BYTES));
+        const bool use_stream = h->stream_kernel && nqb <= 64 && stages >= 4;
+        const size_t stream_smem = static_cast<size_t>(std::max(stages, 0)) * STREAM_X_STAGE_BYTES + q_bytes + STREAM_MISC_BYTES;
         if (use_stream) CAP_RC(make_tmap_bf16(h, &tmap_q, h->q16.p, pad_q(nqb), h->d_pad, nq_s));
-        // ... and the whole slab schedule in one launch (stream_search.cuh) when it is known up
-        // front (it is for <= 2048 queries), has at most STREAM_MAX_SLABS slabs, and the in-kernel
-        // refresh's staging fits next to >= 4 corpus stages
-        const int fused_stages = static_cast<int>(std::min<long long>(
-            std::min(STREAM_MAX_STAGES, h->stream_stages),
-            (static_cast<long long>(MAX_SMEM_OPTIN) - STREAM_MISC_BYTES - STREAM_REFRESH_BYTES - static_cast<long long>(q_bytes)) / STREAM_X_STAGE_BYTES));
-        StreamSearchParams ssp{};
-        bool fused_stream = use_stream && h->stream_fused && !h->dbg && fused_stages >= 4 && nqb <= h->sm_count;
-        if (fused_stream) {
-            std::vector<int64_t> sizes;
-            plan_fixed_slabs(n, slab, cap, k, &sizes);
-            if (sizes.empty() || sizes.size() > static_cast<size_t>(STREAM_MAX_SLABS)) {
-                fused_stream = false;
-            } else {
-                ssp.n_slabs = static_cast<int>(sizes.size());
-                ssp.slab_row[0] = 0;
-                for (size_t i = 0; i < sizes.size(); i++) ssp.slab_row[i + 1] = ssp.slab_row[i] + sizes[i];
-                CAP_RC(ensure(h, h->stream_sync, STREAM_SYNC_WORDS * sizeof(unsigned int)));
-            }
-        }
         // Threshold bootstrap (latency regime, streaming kernel): the geometric schedule spends two
         // dependent rounds (dense slab -> refresh -> small slab -> refresh) before the main slab may
         // start.  Instead: ONE group-max launch over a sample of boot_tiles tiles spread evenly
@@ -880,7 +826,7 @@ int tensor_search(b2ip_handle h, const float* q32, int64_t nq, int k, float* d_s
         // part of the corpus (k <= 42 at the default capacity).
         int boot_grid = 0;
         int64_t boot_tiles = 0;
-        if (use_stream && !fused_stream && h->bootstrap && !h->dbg && n > slab)
+        if (use_stream && h->bootstrap && !h->dbg && n > slab)
             plan_bootstrap(n, k, cap, h->sm_count, h->d_pad, h->bootstrap_max_mb, &boot_grid, &boot_tiles);
         const bool bootstrap = boot_grid > 0;
         if (bootstrap) CAP_RC(ensure(h, h->gmax, static_cast<size_t>(nq_s) * boot_grid * STREAM_TILE_X * sizeof(uint32_t)));
@@ -889,8 +835,7 @@ int tensor_search(b2ip_handle h, const float* q32, int64_t nq, int k, float* d_s
             reinterpret_cast<float*>(h->eps2.p), reinterpret_cast<float*>(h->thr.p),
             reinterpret_cast<int*>(h->cnt.p), reinterpret_cast<int*>(h->kept.p),
             reinterpret_cast<int*>(h->flags.p), h->sh, nq_pad, h->gstats,
-            dense_first && !bootstrap ? static_cast<int>(first_slab) : 0, dyn,
-            fused_stream ? reinterpret_cast<unsigned int*>(h->stream_sync.p) : nullptr);
+            dense_first && !bootstrap ? static_cast<int>(first_slab) : 0, dyn);
         h->stats.total_launches++;
 
         CoarseParams cp{};
@@ -936,10 +881,10 @@ int tensor_search(b2ip_handle h, const float* q32, int64_t nq, int k, float* d_s
             CAP_TRY(rec(e0));
             if (nq_s == 32)
                 coarse_stream_kernel<32, true><<<boot_grid, COARSE_THREADS, stream_smem, h->stream>>>(
-                    tmap_q, tmap_x_pair, cp, stream_stages);
+                    tmap_q, tmap_x_pair, cp, stages);
             else
                 coarse_stream_kernel<64, true><<<boot_grid, COARSE_THREADS, stream_smem, h->stream>>>(
-                    tmap_q, tmap_x_pair, cp, stream_stages);
+                    tmap_q, tmap_x_pair, cp, stages);
             CAP_TRY(rec(e1));
             bootstrap_threshold_kernel<<<nqb, SEL_THREADS, static_cast<size_t>(boot_grid) * STREAM_TILE_X * sizeof(uint32_t), h->stream>>>(
                 reinterpret_cast<const uint32_t*>(h->gmax.p), boot_grid * STREAM_TILE_X, k,
@@ -959,7 +904,6 @@ int tensor_search(b2ip_handle h, const float* q32, int64_t nq, int k, float* d_s
             s = std::min<int64_t>(s, std::max<int64_t>(1, (1ll << 30) / std::max(1, cp.q_tiles)) * STREAM_TILE_X);
             if (done + s < n) s = std::max<int64_t>(TILE_X, s / TILE_X * TILE_X);
             s = std::min<int64_t>(s, n - done);
-            if (fused_stream) s = n;             // every slab of the schedule in this one launch
             cp.x_row0 = done;
             cp.x_row_end = done + s;
             cp.x_tiles = use_stream ? static_cast<int>((s + STREAM_TILE_X - 1) / STREAM_TILE_X)
@@ -969,58 +913,14 @@ int tensor_search(b2ip_handle h, const float* q32, int64_t nq, int k, float* d_s
             const long long tiles = static_cast<long long>(cp.q_tiles) * cp.x_tiles;
             cudaEvent_t e0 = get_event(h, ev_used++), e1 = get_event(h, ev_used++);
             CAP_TRY(rec(e0));
-            if (fused_stream) {
-                long long max_tiles = 1;
-                for (int i = 0; i < ssp.n_slabs; i++)
-                    max_tiles = std::max<long long>(max_tiles, (ssp.slab_row[i + 1] - ssp.slab_row[i] + STREAM_TILE_X - 1) / STREAM_TILE_X);
-                // the first nqb CTAs refresh one query each between slabs: the grid holds at least that many
-                const int grid = static_cast<int>(std::min<long long>(std::max<long long>(max_tiles, nqb), h->sm_count));
-                ssp.dense_first = dense_first ? 1 : 0;
-                ssp.k = k;
-                ssp.thr = reinterpret_cast<float*>(h->thr.p);
-                ssp.kept = reinterpret_cast<int*>(h->kept.p);
-                ssp.eps2 = reinterpret_cast<const float*>(h->eps2.p);
-                ssp.flags = reinterpret_cast<int*>(h->flags.p);
-                ssp.gstats = h->gstats;
-                ssp.sync = reinterpret_cast<unsigned int*>(h->stream_sync.p);
-                ssp.timeout_ns = h->stream_timeout_ns;
-                cp.x_tiles = static_cast<int>(max_tiles);
-                // cooperative launch: the CTAs wait for each other between slabs, so the grid must be
-                // co-resident even when another stream / process shares the GPU
-                cudaLaunchConfig_t cfg{};
-                cfg.gridDim = dim3(static_cast<unsigned int>(grid));
-                cfg.blockDim = dim3(COARSE_THREADS);
-                cfg.dynamicSmemBytes = static_cast<size_t>(fused_stages) * STREAM_X_STAGE_BYTES + q_bytes +
-                                       STREAM_MISC_BYTES + STREAM_REFRESH_BYTES;
-                cfg.stream = h->stream;
-                cudaLaunchAttribute at[1];
-                at[0].id = cudaLaunchAttributeCooperative;
-                at[0].val.cooperative = 1;
-                cfg.attrs = at;
-                cfg.numAttrs = h->stream_coop ? 1 : 0;
-                const cudaError_t le =
-                    nq_s == 32 ? cudaLaunchKernelEx(&cfg, coarse_stream_search_kernel<32>, tmap_q, tmap_x_pair, cp, ssp, fused_stages)
-                               : cudaLaunchKernelEx(&cfg, coarse_stream_search_kernel<64>, tmap_q, tmap_x_pair, cp, ssp, fused_stages);
-                if (le != cudaSuccess) {
-                    // not launchable here (e.g. an SM partition smaller than the grid): per-slab launches from now on
-                    abort_capture();
-                    cudaGetLastError();
-                    if (h->verbose) fprintf(stderr, "[b2ip] one-launch streaming search unavailable (%s): per-slab launches\n", cudaGetErrorString(le));
-                    h->stream_fused = 0;
-                    h->opt_gen++;
-                    CU_TRY(h, cudaStreamSynchronize(h->stream));
-                    memset(&h->stats, 0, sizeof(h->stats));
-                    h->stats.nq = nq; h->stats.ntotal = h->n; h->stats.k = k; h->stats.mode_used = B2IP_MODE_TENSOR;
-                    return tensor_search(h, q32, nq, k, d_scores, d_rows);
-                }
-            } else if (use_stream) {
+            if (use_stream) {
                 const int grid = static_cast<int>(std::min<long long>(cp.x_tiles, h->sm_count));
                 if (nq_s == 32)
                     coarse_stream_kernel<32><<<grid, COARSE_THREADS, stream_smem, h->stream>>>(
-                        tmap_q, tmap_x_pair, cp, stream_stages);
+                        tmap_q, tmap_x_pair, cp, stages);
                 else
                     coarse_stream_kernel<64><<<grid, COARSE_THREADS, stream_smem, h->stream>>>(
-                        tmap_q, tmap_x_pair, cp, stream_stages);
+                        tmap_q, tmap_x_pair, cp, stages);
             } else if (use_pair) {
                 const int grid = 2 * static_cast<int>(std::min<long long>(tiles, h->sm_count / 2));
                 coarse_filter_pair_kernel<<<grid, COARSE_THREADS, PAIR_SMEM_BYTES, h->stream>>>(
@@ -1051,7 +951,7 @@ int tensor_search(b2ip_handle h, const float* q32, int64_t nq, int k, float* d_s
             CAP_TRY(rec(e2));
             h->stats.coarse_launches++;
             h->stats.total_launches += fused ? 1 : 2;
-            h->stats.slabs += fused_stream ? ssp.n_slabs : 1;
+            h->stats.slabs++;
             h->stats.coarse_flops += 2.0 * nqb * static_cast<double>(s) * h->d;
             done += s;
             if (last) break;
@@ -1381,8 +1281,6 @@ int b2ip_create_ex(int d, int device, int store_dtype, b2ip_handle* out) {
             cudaFuncSetAttribute(coarse_stream_kernel<32, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, MAX_SMEM_OPTIN) != cudaSuccess ||
             cudaFuncSetAttribute(coarse_stream_kernel<64, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, MAX_SMEM_OPTIN) != cudaSuccess ||
             cudaFuncSetAttribute(bootstrap_threshold_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, BOOT_MAX_GROUPS * 4) != cudaSuccess ||
-            cudaFuncSetAttribute(coarse_stream_search_kernel<32>, cudaFuncAttributeMaxDynamicSharedMemorySize, MAX_SMEM_OPTIN) != cudaSuccess ||
-            cudaFuncSetAttribute(coarse_stream_search_kernel<64>, cudaFuncAttributeMaxDynamicSharedMemorySize, MAX_SMEM_OPTIN) != cudaSuccess ||
             cudaFuncSetAttribute(finalize_kernel<true, ROWS_F32>, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(fin_smem)) != cudaSuccess ||
             cudaFuncSetAttribute(finalize_kernel<true, ROWS_BF16>, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(fin_smem)) != cudaSuccess ||
             cudaFuncSetAttribute(finalize_kernel<true, ROWS_F16>, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(fin_smem)) != cudaSuccess ||
@@ -1395,7 +1293,6 @@ int b2ip_create_ex(int d, int device, int store_dtype, b2ip_handle* out) {
                                             // the corpus tiles of a group stay L2 resident (measured best)
     if (const char* s = getenv("B2IP_GX")) h->gx = std::max(1, atoi(s));
     if (const char* s = getenv("B2IP_STREAM_KERNEL")) h->stream_kernel = atoi(s);
-    if (const char* s = getenv("B2IP_STREAM_FUSED")) h->stream_fused = atoi(s);
     if (const char* s = getenv("B2IP_BOOTSTRAP")) h->bootstrap = atoi(s);
     if (const char* s = getenv("B2IP_BOOTSTRAP_MAX_MB")) h->bootstrap_max_mb = std::max(0, atoi(s));
     if (const char* s = getenv("B2IP_HINT_Q")) h->hint_q = atoi(s);
@@ -1414,7 +1311,7 @@ void b2ip_destroy(b2ip_handle h) {
     if (h->own_stream) cudaStreamSynchronize(h->own_stream);
     for (DevBuf* b : {&h->q16, &h->eps2, &h->thr, &h->cnt, &h->kept, &h->flags, &h->cand, &h->qstage, &h->qhalf,
                       &h->out_s, &h->out_r, &h->exact_scores, &h->exact_misc, &h->qlist, &h->stage,
-                      &h->seg_tab, &h->stream_sync, &h->gmax})
+                      &h->seg_tab, &h->gmax})
         release(*b);
     if (h->v16.base || h->v32.base) {
         vmm_free(h, h->v32);
@@ -1468,11 +1365,7 @@ int b2ip_set_option(b2ip_handle h, const char* name, int64_t value) {
     else if (n == "bootstrap") h->bootstrap = static_cast<int>(value);
     else if (n == "bootstrap_max_mb") h->bootstrap_max_mb = static_cast<int>(std::min<int64_t>(std::max<int64_t>(0, value), 1 << 20));
     else if (n == "stream_kernel") h->stream_kernel = static_cast<int>(value);
-    else if (n == "stream_fused") h->stream_fused = static_cast<int>(value);
-    else if (n == "stream_coop") h->stream_coop = static_cast<int>(value);
     else if (n == "list_fill_pct") h->list_fill_pct = std::min(90, std::max(10, static_cast<int>(value)));
-    else if (n == "stream_stages") h->stream_stages = std::max(4, static_cast<int>(value));
-    else if (n == "stream_timeout_ms") h->stream_timeout_ns = std::max<int64_t>(1, value) * 1000000ll;
     else if (n == "fuse_refresh") h->fuse_refresh = static_cast<int>(value);
     else if (n == "two_stage") h->two_stage = static_cast<int>(value);
     else if (n == "cand_budget_mb") h->cand_budget_bytes = std::max<int64_t>(1, value) << 20;

@@ -511,7 +511,8 @@ coarse_filter_pair_kernel(const __grid_constant__ CUtensorMap tmap_q,
 //                     per-query thresholds held in registers
 // =======================================================================================
 constexpr int STREAM_TILE_X = 128;
-constexpr int STREAM_MAX_STAGES = 12;
+constexpr int STREAM_MAX_STAGES = 12;   // corpus stages the barrier area holds
+constexpr int STREAM_STAGES = 8;        // stages run when they fit (5 - 12 measure the same: DESIGN 4.1d)
 constexpr int STREAM_ACC = 4;
 constexpr int STREAM_X_STAGE_BYTES = STREAM_TILE_X * KBLOCK_BYTES;   // 16 KiB
 constexpr int STREAM_MISC_BYTES = 1024 /*align*/ + 320 /*barriers*/;

@@ -264,15 +264,11 @@ __global__ void prep_queries_kernel(const float* __restrict__ q32, __nv_bfloat16
                                     int* __restrict__ cnt, int* __restrict__ kept,
                                     int* __restrict__ flags, int sh, int nq_pad,
                                     long long* __restrict__ gstats, int init_cnt,
-                                    const DynArgs* __restrict__ dyn,
-                                    unsigned int* __restrict__ stream_sync = nullptr) {
+                                    const DynArgs* __restrict__ dyn) {
     if (dyn) q32 = dyn->q32;
     const int lane = threadIdx.x & 31;
     const int q = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;
     if (blockIdx.x == 0 && threadIdx.x < GS_COUNT && gstats) gstats[threadIdx.x] = 0;
-    // arrival counter, abort word and per-query threshold epochs of the one-launch streaming search
-    if (stream_sync && blockIdx.x == 0)
-        for (int i = threadIdx.x; i < 2 + 64; i += blockDim.x) stream_sync[i] = 0u;
     if (q >= nq) {
         // rows that pad the last (pair) tile: zeros, so no TMA box hangs over the tensor's end
         if (q < nq_pad) {
@@ -317,27 +313,6 @@ __global__ void prep_queries_kernel(const float* __restrict__ q32, __nv_bfloat16
 }
 
 // ---------------------------------------------------------------------------------------
-// thread groups the selection routines run on
-// ---------------------------------------------------------------------------------------
-// The whole CTA (refresh / finalize kernels), or a contiguous range of its warps on a named
-// barrier: the four epilogue warps of the multi-slab streaming kernel (stream_search.cuh) refresh
-// the thresholds between slabs while the TMA and MMA warps of the same CTA keep streaming.
-struct CtaGroup {
-    static __device__ __forceinline__ int tid() { return static_cast<int>(threadIdx.x); }
-    static __device__ __forceinline__ int size() { return static_cast<int>(blockDim.x); }
-    static __device__ __forceinline__ void sync() { __syncthreads(); }
-};
-template <int kFirstThread, int kThreads, int kBarrier>
-struct WarpRangeGroup {
-    static_assert(kFirstThread % 32 == 0 && kThreads % 32 == 0 && kThreads <= SEL_THREADS && kBarrier > 0, "whole warps");
-    static __device__ __forceinline__ int tid() { return static_cast<int>(threadIdx.x) - kFirstThread; }
-    static __device__ __forceinline__ int size() { return kThreads; }
-    static __device__ __forceinline__ void sync() {
-        asm volatile("bar.sync %0, %1;" ::"n"(kBarrier), "n"(kThreads) : "memory");
-    }
-};
-
-// ---------------------------------------------------------------------------------------
 // block-wide radix select
 // ---------------------------------------------------------------------------------------
 // Top `n_bytes` bytes of the k-th largest of keys[0..n) (1 <= k <= n); low bytes are zero.
@@ -346,22 +321,22 @@ struct WarpRangeGroup {
 // mantissa bits (the bound is at most 2^-15 relative below the true value, ~1/500 of the error
 // margin it is combined with) and saves a pass.  first_pass / prefix0: leading bytes all keys are
 // known to share (see common_prefix_bytes) are not counted again.
-template <class G = CtaGroup>
 __device__ unsigned long long block_radix_select(const unsigned long long* __restrict__ keys,
                                                  int n, int k, int n_bytes, unsigned int* hist,
                                                  unsigned long long* s_prefix, int* s_krem,
                                                  int first_pass = 0, unsigned long long prefix0 = 0ull) {
+    const int tid = threadIdx.x, nt = blockDim.x;
     unsigned long long prefix = prefix0;
     int krem = k;
     for (int pass = first_pass; pass < n_bytes; pass++) {
         const int shift = 56 - 8 * pass;
-        for (int i = G::tid(); i < 256; i += G::size()) hist[i] = 0;
-        G::sync();
+        for (int i = tid; i < 256; i += nt) hist[i] = 0;
+        __syncthreads();
         const unsigned long long mask = pass == 0 ? 0ull : (~0ull << (shift + 8));
         // Scores of one list share their leading bytes, so most lanes of a warp hit the SAME bin:
         // lanes with equal digits elect one of them to add the whole group's count.
-        for (int base = 0; base < n; base += G::size()) {
-            const int i = base + G::tid();
+        for (int base = 0; base < n; base += nt) {
+            const int i = base + tid;
             unsigned int digit = 256u;                       // 256 = not counted
             if (i < n) {
                 const unsigned long long key = keys[i];
@@ -371,15 +346,15 @@ __device__ unsigned long long block_radix_select(const unsigned long long* __res
             // counted by lane 0 in one add, the rest add for themselves
             const unsigned int first = __shfl_sync(0xffffffffu, digit, 0);
             const unsigned int same = __ballot_sync(0xffffffffu, digit == first);
-            if ((G::tid() & 31) == 0) {
+            if ((tid & 31) == 0) {
                 if (digit < 256u) atomicAdd(&hist[digit], static_cast<unsigned int>(__popc(same)));
             } else if (digit < 256u && digit != first) {
                 atomicAdd(&hist[digit], 1u);
             }
         }
-        G::sync();
-        if (G::tid() < 32) {
-            const int lane = G::tid();
+        __syncthreads();
+        if (tid < 32) {
+            const int lane = tid;
             unsigned int c[8], sum = 0;
 #pragma unroll
             for (int j = 0; j < 8; j++) { c[j] = hist[255 - (8 * lane + j)]; sum += c[j]; }
@@ -402,7 +377,7 @@ __device__ unsigned long long block_radix_select(const unsigned long long* __res
                 *s_krem = static_cast<int>(r);
             }
         }
-        G::sync();
+        __syncthreads();
         prefix = *s_prefix;
         krem = *s_krem;
     }
@@ -419,29 +394,30 @@ __device__ unsigned long long block_radix_select(const unsigned long long* __res
 // hist: BOUND_BINS words.  Ends with a barrier; s_prefix / s_krem / s_warp are free afterwards.
 // K = u64 keys (score word on top) or bare u32 score words; entries whose score word is below kmin
 // are not counted (bootstrap_threshold_kernel: empty groups hold 0), so k counts the others.
+// Written for a block of 128 or 256 threads; every caller runs SEL_THREADS = 256.
 constexpr int BOUND_BINS = 1024;
 
 __device__ __forceinline__ uint32_t score_word(unsigned long long key) { return static_cast<uint32_t>(key >> 32); }
 __device__ __forceinline__ uint32_t score_word(uint32_t word) { return word; }
 
-template <class G = CtaGroup, class K = unsigned long long>
+template <class K = unsigned long long>
 __device__ uint32_t block_bound_select(const K* skeys, int n, int k, uint32_t kmin,
                                        uint32_t kmax, unsigned int* hist,
                                        unsigned long long* s_prefix, int* s_krem, int* s_warp) {
     if (kmin == kmax) return kmin;
     const uint32_t range = kmax - kmin;
     const int shift = max(0, 32 - __clz(static_cast<int>(range)) - 10);     // (range >> shift) < BOUND_BINS
-    const int tid = G::tid(), nt = G::size();
+    const int tid = threadIdx.x, nt = blockDim.x;
     const int lane = tid & 31, warp = tid >> 5;
     for (int i = tid; i < BOUND_BINS; i += nt) hist[i] = 0;
-    G::sync();
+    __syncthreads();
     for (int i = tid; i < n; i += nt) {
         const uint32_t hi = score_word(skeys[i]);
         if (hi >= kmin) atomicAdd(&hist[(hi - kmin) >> shift], 1u);
     }
-    G::sync();
+    __syncthreads();
     // thread t owns the `per` bins just below BOUND_BINS - per * t: the top bins come first
-    const int per = BOUND_BINS / nt;                     // 4 (256 threads) or 8 (128 threads)
+    const int per = BOUND_BINS / nt;                     // 4 (SEL_THREADS = 256) or 8 (128 threads)
     const int top = BOUND_BINS - 1 - per * tid;
     unsigned int c[8], sum = 0;
 #pragma unroll
@@ -456,7 +432,7 @@ __device__ uint32_t block_bound_select(const K* skeys, int n, int k, uint32_t km
         if (lane >= o) incl += t;
     }
     if (lane == 31) s_warp[warp] = static_cast<int>(incl);
-    G::sync();
+    __syncthreads();
     for (int w = 0; w < warp; w++) incl += static_cast<unsigned int>(s_warp[w]);
     const unsigned int excl = incl - sum;
     if (excl < static_cast<unsigned int>(k) && static_cast<unsigned int>(k) <= incl) {
@@ -471,11 +447,11 @@ __device__ uint32_t block_bound_select(const K* skeys, int n, int k, uint32_t km
         *s_krem = static_cast<int>(r);
     }
     for (int i = tid; i < 256; i += nt) hist[i] = 0;     // (every thread has read its bins)
-    G::sync();
+    __syncthreads();
     const int bin = static_cast<int>(*s_prefix);
     const int krem = *s_krem;
     uint32_t bound = kmin + (static_cast<uint32_t>(bin) << shift);
-    if (shift == 0) { G::sync(); return bound; }
+    if (shift == 0) { __syncthreads(); return bound; }
     // split that bin into 256 (or 2^shift) sub-bins
     const int sub_shift = max(0, shift - 8);
     for (int i = tid; i < n; i += nt) {
@@ -484,7 +460,7 @@ __device__ uint32_t block_bound_select(const K* skeys, int n, int k, uint32_t km
         if (w >= kmin && static_cast<int>(off >> shift) == bin)
             atomicAdd(&hist[(off - (static_cast<uint32_t>(bin) << shift)) >> sub_shift], 1u);
     }
-    G::sync();
+    __syncthreads();
     if (tid < 32) {
         unsigned int d[8], dsum = 0;
 #pragma unroll
@@ -507,21 +483,21 @@ __device__ uint32_t block_bound_select(const K* skeys, int n, int k, uint32_t km
             s_warp[0] = digit;
         }
     }
-    G::sync();
+    __syncthreads();
     bound += static_cast<uint32_t>(s_warp[0]) << sub_shift;
-    G::sync();                                           // s_warp is free again
+    __syncthreads();                                     // s_warp is free again
     return bound;
 }
 
 // In-place stream compaction of keys[0..n): keeps keys whose high word is > hi_thr
 // (or, with by_key, keys >= key_thr).  Returns the number kept (all threads).
-template <class G = CtaGroup>
 __device__ int block_compact(const unsigned long long* keys, int n, bool by_key, uint32_t hi_thr,
                              unsigned long long key_thr, unsigned long long* out, int* s_warp) {
-    const int lane = G::tid() & 31, warp = G::tid() >> 5, nw = G::size() >> 5;
+    const int tid = threadIdx.x, nt = blockDim.x;
+    const int lane = tid & 31, warp = tid >> 5, nw = nt >> 5;
     int base_out = 0;
-    for (int base = 0; base < n; base += G::size()) {
-        const int i = base + G::tid();
+    for (int base = 0; base < n; base += nt) {
+        const int i = base + tid;
         unsigned long long key = 0;
         bool keep = false;
         if (i < n) {
@@ -530,7 +506,7 @@ __device__ int block_compact(const unsigned long long* keys, int n, bool by_key,
         }
         const unsigned int ballot = __ballot_sync(0xffffffffu, keep);
         if (lane == 0) s_warp[warp] = __popc(ballot);
-        G::sync();
+        __syncthreads();
         int off = 0, tot = 0;
         for (int w = 0; w < nw; w++) {
             const int c = s_warp[w];
@@ -539,18 +515,18 @@ __device__ int block_compact(const unsigned long long* keys, int n, bool by_key,
         }
         if (keep) out[base_out + off + __popc(ballot & ((1u << lane) - 1u))] = key;
         base_out += tot;
-        G::sync();
+        __syncthreads();
     }
     return base_out;
 }
 
 // Same selection, for `out` NOT aliasing `keys`: each warp owns a contiguous segment, one
 // counting pass, one block barrier, one writing pass (2 barriers instead of 2 per 256 keys).
-template <class G = CtaGroup>
 __device__ int block_compact_disjoint(const unsigned long long* keys, int n, bool by_key,
                                       uint32_t hi_thr, unsigned long long key_thr,
                                       unsigned long long* out, int* s_warp, bool invert = false) {
-    const int lane = G::tid() & 31, warp = G::tid() >> 5, nw = G::size() >> 5;
+    const int tid = threadIdx.x, nt = blockDim.x;
+    const int lane = tid & 31, warp = tid >> 5, nw = nt >> 5;
     const int seg = ((n + nw - 1) / nw + 31) & ~31;
     const int b = warp * seg, e = min(n, b + seg);
     int mine = 0;
@@ -565,7 +541,7 @@ __device__ int block_compact_disjoint(const unsigned long long* keys, int n, boo
         mine += __popc(__ballot_sync(0xffffffffu, keep));
     }
     if (lane == 0) s_warp[warp] = mine;
-    G::sync();
+    __syncthreads();
     int off = 0, tot = 0;
     for (int w = 0; w < nw; w++) {
         const int c = s_warp[w];
@@ -585,7 +561,7 @@ __device__ int block_compact_disjoint(const unsigned long long* keys, int n, boo
         if (keep) out[off + __popc(ballot & ((1u << lane) - 1u))] = key;
         off += __popc(ballot);
     }
-    G::sync();
+    __syncthreads();
     return tot;
 }
 
@@ -596,23 +572,23 @@ __device__ int block_compact_disjoint(const unsigned long long* keys, int n, boo
 // so every member of the final exact top-k has exact >= c_k - eps and coarse >= c_k - 2 eps:
 // rows below that can be dropped for good, and later slabs only need to report above it.
 // Returns the number of entries the list holds afterwards (block-uniform), or -1 when the query
-// overflowed its list (flagged for the exact path).  `scratch` = `scratch_keys` keys of
+// overflowed its list (flagged for the exact path).  `scratch` = REFRESH_SMEM_KEYS keys of
 // shared memory: lists that fit are pulled into it once, so the select passes and the
-// compaction never touch L2 again.  G = the threads that run it (see CtaGroup).
-template <class G = CtaGroup>
+// compaction never touch L2 again.
 __device__ int refresh_list(int q, int k, int cap, unsigned long long* __restrict__ cand,
                             int* __restrict__ cnt, int* __restrict__ kept, float* __restrict__ thr,
                             const float* __restrict__ eps2, int* __restrict__ flags,
                             long long* __restrict__ gstats, unsigned long long* scratch,
                             unsigned int* hist, unsigned long long* s_prefix, int* s_krem,
-                            int* s_warp, int scratch_keys = REFRESH_SMEM_KEYS) {
+                            int* s_warp) {
     const int n = cnt[q];
     const int prev = kept[q];
-    if (G::tid() == 0) { s_warp[0] = -1; s_warp[1] = 0; }   // min / max of the staged keys' score words
-    G::sync();                                 // everyone has read the counters
+    const int tid = threadIdx.x;
+    if (tid == 0) { s_warp[0] = -1; s_warp[1] = 0; }   // min / max of the staged keys' score words
+    __syncthreads();                                 // everyone has read the counters
     if (n > cap) {
         // more hits than the list holds: this query is re-run on the exact path
-        if (G::tid() == 0) {
+        if (tid == 0) {
             flags[q] |= FLAG_OVERFLOW;
             thr[q] = INFINITY;
             cnt[q] = 0;
@@ -622,22 +598,22 @@ __device__ int refresh_list(int q, int k, int cap, unsigned long long* __restric
         return -1;
     }
     if (n == prev) return n;
-    if (G::tid() == 0)
+    if (tid == 0)
         atomicAdd(reinterpret_cast<unsigned long long*>(gstats + GS_CANDIDATES),
                   static_cast<unsigned long long>(n - prev));
     if (n < k) {
-        if (G::tid() == 0) kept[q] = n;
+        if (tid == 0) kept[q] = n;
         return n;
     }
     unsigned long long* keys = cand + static_cast<long long>(q) * cap;
     const unsigned long long* src = keys;
     uint32_t ck_word;
-    if (n <= scratch_keys) {
+    if (n <= REFRESH_SMEM_KEYS) {
         // the list is staged in shared memory once; its smallest / largest score word, found on the
         // way, span the histogram of the bound select
         unsigned int lo = 0xFFFFFFFFu, hi = 0u;
-        int i = G::tid();
-        const int nt = G::size();
+        int i = tid;
+        const int nt = blockDim.x;
         // four independent loads in flight per thread: this pass is what the kernel waits for
         for (; i + 3 * nt < n; i += 4 * nt) {
             const unsigned long long k0 = keys[i], k1 = keys[i + nt], k2 = keys[i + 2 * nt], k3 = keys[i + 3 * nt];
@@ -655,26 +631,26 @@ __device__ int refresh_list(int q, int k, int cap, unsigned long long* __restric
         }
         lo = __reduce_min_sync(0xffffffffu, lo);
         hi = __reduce_max_sync(0xffffffffu, hi);
-        if ((G::tid() & 31) == 0) {
+        if ((tid & 31) == 0) {
             atomicMin(reinterpret_cast<unsigned int*>(&s_warp[0]), lo);
             atomicMax(reinterpret_cast<unsigned int*>(&s_warp[1]), hi);
         }
-        G::sync();
+        __syncthreads();
         src = scratch;
         const unsigned int kmin = static_cast<unsigned int>(s_warp[0]), kmax = static_cast<unsigned int>(s_warp[1]);
-        G::sync();                             // s_warp is reused by the select and the compaction
-        ck_word = block_bound_select<G>(scratch, n, k, kmin, kmax, hist, s_prefix, s_krem, s_warp);
+        __syncthreads();                             // s_warp is reused by the select and the compaction
+        ck_word = block_bound_select(scratch, n, k, kmin, kmax, hist, s_prefix, s_krem, s_warp);
     } else {
         // lists beyond the staging area (k > 1024): 3-byte radix select out of L2
-        ck_word = static_cast<uint32_t>(block_radix_select<G>(src, n, k, 3, hist, s_prefix, s_krem) >> 32);
+        ck_word = static_cast<uint32_t>(block_radix_select(src, n, k, 3, hist, s_prefix, s_krem) >> 32);
     }
     const float ck = unorder_f32(ck_word);
     float t = __fsub_rd(ck, eps2[q]);
     if (!(t == t)) t = -INFINITY;                    // inf - inf: no usable threshold
     t = nextafterf(t, -INFINITY);                    // admission test is strict
-    const int m = (src == keys) ? block_compact<G>(src, n, false, order_f32(t), 0ull, keys, s_warp)
-                                : block_compact_disjoint<G>(src, n, false, order_f32(t), 0ull, keys, s_warp);
-    if (G::tid() == 0) {
+    const int m = (src == keys) ? block_compact(src, n, false, order_f32(t), 0ull, keys, s_warp)
+                                : block_compact_disjoint(src, n, false, order_f32(t), 0ull, keys, s_warp);
+    if (tid == 0) {
         cnt[q] = m;
         kept[q] = m;
         thr[q] = t;
@@ -839,10 +815,10 @@ bootstrap_threshold_kernel(const uint32_t* __restrict__ gmax, int groups, int k,
         if (static_cast<int>(s_valid) < k) return;           // thr[q] stays -inf (prep_queries_kernel)
         const unsigned int kmin = s_lo, kmax = s_hi;
         __syncthreads();
-        ck_word = block_bound_select<CtaGroup, uint32_t>(s_gmax, groups, k, kmin, kmax, hist,
-                                                         &s_prefix, &s_krem, s_warp);
-        ck_word = block_bound_select<CtaGroup, uint32_t>(s_gmax, groups, k, ck_word, kmax, hist,
-                                                         &s_prefix, &s_krem, s_warp);
+        ck_word = block_bound_select<uint32_t>(s_gmax, groups, k, kmin, kmax, hist,
+                                               &s_prefix, &s_krem, s_warp);
+        ck_word = block_bound_select<uint32_t>(s_gmax, groups, k, ck_word, kmax, hist,
+                                               &s_prefix, &s_krem, s_warp);
     }
     if (tid == 0) {
         float t = __fsub_rd(unorder_f32(ck_word), eps2[q]);

@@ -112,14 +112,11 @@ int b2ip_set_stream(b2ip_handle h, void* cuda_stream);
  * pass instead of bf16 (tighter error bound, saturating at +-65504), "pair" 0/1 CTA-pair kernel,
  * "graph" 0/1 CUDA-graph replay of small-batch searches (env B2IP_GRAPH), "graph_timing" 0/1 keep
  * the per-kernel event records inside the graph (b2ip_stats' coarse_ms etc.), "stream_kernel" 0/1
- * streaming kernel for batches <= 64, "stream_stages" cap on its corpus stages in flight per SM,
- * "stream_fused" 0/1 (env B2IP_STREAM_FUSED, default 0) the whole slab schedule of such a batch in
- * ONE cooperative launch with in-kernel threshold refreshes (same results; measured slower, see
- * DESIGN.md 4.1d), "stream_timeout_ms" bound on its in-kernel waits, "bootstrap" 0/1 (env
- * B2IP_BOOTSTRAP, default 1) first threshold of a batch <= 64 from the group maxima of a corpus
- * sample + ONE filtered slab over all rows instead of the geometric slab schedule, taken while the
- * sample is at most "bootstrap_max_mb" (env B2IP_BOOTSTRAP_MAX_MB, default 64) MiB of 16-bit rows
- * (same results; DESIGN.md 4.1e; b2ip_stats_t.sample_rows tells which schedule ran). */
+ * streaming kernel for batches <= 64, "bootstrap" 0/1 (env B2IP_BOOTSTRAP, default 1) first
+ * threshold of a batch <= 64 from the group maxima of a corpus sample + ONE filtered slab over all
+ * rows instead of the geometric slab schedule, taken while the sample is at most
+ * "bootstrap_max_mb" (env B2IP_BOOTSTRAP_MAX_MB, default 64) MiB of 16-bit rows (same results;
+ * DESIGN.md 4.1e; b2ip_stats_t.sample_rows tells which schedule ran). */
 int b2ip_set_option(b2ip_handle h, const char* name, int64_t value);
 
 /* Optional capacity hint before a series of b2ip_add calls (avoids regrowth copies). */

@@ -1,7 +1,6 @@
-"""Latency regime (BASELINE config 5) A/B on ONE GPU holding one shard: the one-launch streaming
-search (option stream_fused=1, csrc/stream_search.cuh) against the per-slab launch sequence
-(stream_fused=0), and the threshold bootstrap (--bootstrap 1: group-max sample + one filtered slab)
-against the geometric slab schedule (0), all replayed from a CUDA graph.  One JSON line per case."""
+"""Latency regime (BASELINE config 5) A/B on ONE GPU holding one shard: the threshold bootstrap
+(--bootstrap 1: group-max sample + one filtered slab) against the geometric slab schedule (0), both
+replayed from a CUDA graph.  One JSON line per case."""
 import argparse, json, os, sys, time
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path[:0] = [ROOT, os.path.join(ROOT, "czech-contriever_b200")]
@@ -14,9 +13,7 @@ ap.add_argument("--d", type=int, default=768)
 ap.add_argument("--batches", default="1,64")
 ap.add_argument("--k", type=int, default=10)
 ap.add_argument("--iters", type=int, default=300)
-ap.add_argument("--fused", default="0,1,0,1")
-ap.add_argument("--bootstrap", default="1")
-ap.add_argument("--stages", default="12", help="caps on the corpus stages in flight per SM to try (the kernel takes what fits)")
+ap.add_argument("--bootstrap", default="1,0,1,0")
 a = ap.parse_args()
 dev = torch.device("cuda", 0)
 
@@ -34,12 +31,8 @@ qall = torch.randn((64, a.d), generator=g, device=dev)
 qall /= qall.norm(dim=1, keepdim=True)
 floor_ms = a.n_corpus * a.d * 2 / 6551e9 * 1e3
 ref = {}
-for stages, fused, boot in [(int(st_), int(v), int(b)) for st_ in a.stages.split(",") for v in a.fused.split(",")
-                            for b in a.bootstrap.split(",")]:
+for boot in [int(b) for b in a.bootstrap.split(",")]:
     e.set_option("bootstrap", boot)
-    e.set_option("stream_fused", 1 if fused else 0)      # 2 = one launch, not cooperative
-    e.set_option("stream_coop", 0 if fused == 2 else 1)
-    e.set_option("stream_stages", stages)
     for nq in [int(v) for v in a.batches.split(",")]:
         q = qall[:nq].contiguous()
         for _ in range(20):
@@ -64,7 +57,7 @@ for stages, fused, boot in [(int(st_), int(v), int(b)) for st_ in a.stages.split
             same = bool(torch.equal(ref[nq][1], I) and torch.equal(ref[nq][0], D))
         else:
             ref[nq] = (D.clone(), I.clone())
-        print(json.dumps({"fused": fused, "bootstrap": boot, "cand_per_q": round(cand, 1), "rescored_per_q": round(st["rescored"] / nq, 1), "stages_cap": stages, "n": a.n_corpus, "nq": nq, "k": a.k, "ms_per_batch": round(wall, 4),
+        print(json.dumps({"bootstrap": boot, "cand_per_q": round(cand, 1), "rescored_per_q": round(st["rescored"] / nq, 1), "n": a.n_corpus, "nq": nq, "k": a.k, "ms_per_batch": round(wall, 4),
                           "dev_ms": round(dev_ms / a.iters, 4), "floor_ms_16bit": round(floor_ms, 4),
                           "frac_of_floor": round(floor_ms / wall, 4), "graph_mode": st["graph_mode"],
                           "launches": st["total_launches"], "coarse_launches": st["coarse_launches"], "slabs": st["slabs"],
