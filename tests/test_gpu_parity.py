@@ -803,11 +803,15 @@ def test_non_finite_values_follow_faiss(fo, store, shadow):
 @pytest.mark.parametrize("d,nq", [(2048, 8), (1024, 40), (1024, 20), (64, 64)])
 def test_small_batches_across_dimensions(fo, d, nq):
     """Batches <= 64 take the streaming kernel (queries resident in shared memory) when the padded
-    batch fits next to >= 4 corpus stages, the single-CTA kernel otherwise (d = 2048 here)."""
+    batch (32 query rows for <= 32 queries, else 64) fits next to >= 4 corpus stages of 16 KiB:
+    d_pad <= 2560 for <= 32 queries, d_pad <= 1280 for 33-64.  All four cases here stream (d = 2048
+    with 8 queries: 128 KiB of queries, 6 stages), which the threshold bootstrap's sample shows; the
+    single-CTA side of the rule is tested by test_gpu_edges.test_small_batch_kernel_choice."""
     x = synth(30_000, d, 141)
     q = synth(nq, d, 142)
     e = _engine(x)
     D, I = e.search(q, 10)
     assert e.stats()["fallback_queries"] == 0 and e.stats()["slabs"] >= 2
+    assert e.stats()["sample_rows"] > 0
     Do, Io = fo.search(q, x, 10)
     fo.compare_topk(D, I, Do, Io, q, x, rtol=RTOL)
