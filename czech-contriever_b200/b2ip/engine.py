@@ -178,6 +178,45 @@ class Engine:
                                        m, MEM_HOST), self._h)
         return D, I
 
+    def range_search(self, queries, radius: float, mode: str = "auto"):
+        """faiss `IndexFlatIP.range_search`: (lims [nq+1] int64, D [total] float32, I [total] int64);
+        query i's hits are D/I[lims[i]:lims[i+1]], every row scoring strictly above `radius`, in
+        ascending row order.  numpy in -> numpy out; torch CUDA tensor in -> CUDA tensors out."""
+        m = _MODES[mode]
+        if _is_torch(queries):
+            import torch
+            assert queries.is_cuda and queries.device.index == self.device
+            q = queries.contiguous() if queries.dtype in (torch.float16, torch.float32) \
+                else queries.float().contiguous()
+            assert q.dim() == 2 and q.shape[1] == self.d, tuple(q.shape)
+            lims = np.empty(q.shape[0] + 1, dtype=np.int64)
+            self._order_after_torch()
+            check(self._lib.b2ip_range_search(self._h, q.shape[0], ctypes.c_void_p(q.data_ptr()),
+                                              B2IP_F16 if q.dtype == torch.float16 else B2IP_F32, float(radius), m,
+                                              MEM_DEVICE, ctypes.c_void_p(lims.ctypes.data)), self._h)
+            total = int(lims[-1])
+            D = torch.empty(total, dtype=torch.float32, device=q.device)
+            I = torch.empty(total, dtype=torch.int64, device=q.device)
+            check(self._lib.b2ip_range_fetch(self._h, ctypes.c_void_p(D.data_ptr()), ctypes.c_void_p(I.data_ptr()),
+                                             MEM_DEVICE), self._h)
+            return torch.from_numpy(lims).to(q.device), D, I
+        q = np.asarray(queries)
+        if q.dtype not in (np.float16, np.float32):
+            q = q.astype(np.float32)
+        q = np.ascontiguousarray(q)
+        if q.ndim != 2 or q.shape[1] != self.d:
+            raise ValueError(f"expected [nq,{self.d}] queries, got {q.shape}")
+        lims = np.empty(q.shape[0] + 1, dtype=np.int64)
+        check(self._lib.b2ip_range_search(self._h, q.shape[0], ctypes.c_void_p(q.ctypes.data),
+                                          B2IP_F16 if q.dtype == np.float16 else B2IP_F32, float(radius), m,
+                                          MEM_HOST, ctypes.c_void_p(lims.ctypes.data)), self._h)
+        total = int(lims[-1])
+        D = np.empty(total, dtype=np.float32)
+        I = np.empty(total, dtype=np.int64)
+        check(self._lib.b2ip_range_fetch(self._h, ctypes.c_void_p(D.ctypes.data), ctypes.c_void_p(I.ctypes.data),
+                                         MEM_HOST), self._h)
+        return lims, D, I
+
     def enable_peer_access(self, peer_device: int) -> None:
         """Kernels of this engine's GPU may store into memory of `peer_device` (same process)."""
         check(self._lib.b2ip_enable_peer_access(self._h, int(peer_device)), self._h)

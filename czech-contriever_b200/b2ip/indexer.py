@@ -159,6 +159,32 @@ class Indexer(object):
             result.extend(map_ids(ids, indexes, indexes.shape[0], indexes.shape[1], list(scores)))
         return result
 
+    def search_range(self, query_vectors, radius: float) -> List[Tuple[List[object], np.ndarray]]:
+        """Every indexed passage whose inner product with the query is strictly above `radius`
+        (faiss `IndexFlatIP.range_search`).  Takes what `search_knn` takes and returns one tuple
+        per query, like `search_knn`: (external ids as `str`, float32 scores), score-descending,
+        equal scores in insertion order."""
+        q = query_vectors
+        if _is_torch(q):
+            q = q.detach()
+            if not q.is_cuda:
+                q = q.numpy()
+        if not _is_torch(q):
+            q = np.asarray(q)
+            if q.dtype not in (np.float16, np.float32):
+                q = q.astype('float32')
+        if len(q) == 0:
+            return []
+        lims, D, I = self.index.range_search(q, radius)
+        if _is_torch(lims):
+            lims, D, I = lims.cpu().numpy(), D.cpu().numpy(), I.cpu().numpy()
+        ids = self.index_id_to_db_id
+        qi = np.repeat(np.arange(len(lims) - 1), np.diff(lims))
+        order = np.lexsort((I, -D.astype(np.float64), qi))
+        D, I = D[order], I[order]
+        return [([str(ids[r]) for r in I[lims[i]:lims[i + 1]].tolist()], D[lims[i]:lims[i + 1]])
+                for i in range(len(lims) - 1)]
+
     def serialize(self, dir_path):
         index_file = os.path.join(dir_path, 'index.faiss')
         meta_file = os.path.join(dir_path, 'index_meta.faiss')

@@ -97,6 +97,22 @@ def level_split(totals: Sequence[int], n: int) -> List[int]:
     return out
 
 
+def merge_range_results(parts):
+    """Merge per-shard range search answers [(lims [nq+1], D [total], I [total]), ...] (global
+    rows, ascending per query) into one: per query, the union of the shards' hits in ascending row
+    order.  Shards hold interleaved row segments, so this is a per-query merge, not a concatenation."""
+    parts = [(np.asarray(l, np.int64), np.asarray(d, np.float32), np.asarray(i, np.int64)) for l, d, i in parts]
+    nq = len(parts[0][0]) - 1
+    qs = [np.repeat(np.arange(nq, dtype=np.int64), np.diff(l)) for l, _, _ in parts]
+    q = np.concatenate(qs)
+    D = np.concatenate([d[:l[-1]] for l, d, _ in parts])
+    I = np.concatenate([i[:l[-1]] for l, _, i in parts])
+    order = np.lexsort((I, q))
+    lims = np.zeros(nq + 1, dtype=np.int64)
+    np.cumsum(np.bincount(q, minlength=nq), out=lims[1:])
+    return lims, D[order], I[order]
+
+
 class MultiGpuEngine:
     def __init__(self, d: int, devices: Optional[Sequence[int]] = None, store: str = "f32",
                  shadow: Optional[str] = None):
@@ -372,6 +388,36 @@ class MultiGpuEngine:
         self.engines[0].download(D.contiguous(), host_out[0])
         self.engines[0].download(I.contiguous(), host_out[1])
         return host_out
+
+    def _range_one(self, g: int, queries, radius: float, mode: str):
+        torch = self._torch
+        dev = torch.device("cuda", self.devices[g])
+        with torch.cuda.device(dev):
+            q = queries
+            if type(q).__module__.startswith("torch") and q.device != dev:
+                q = q.to(dev)
+            lims, D, I = self.engines[g].range_search(q, radius, mode=mode)
+            if type(lims).__module__.startswith("torch"):
+                lims, D, I = lims.cpu().numpy(), D.cpu().numpy(), I.cpu().numpy()
+            st = self.engines[g].stats()
+        return (lims, D, I), st
+
+    def range_search(self, queries, radius: float, mode: str = "auto"):
+        """One range search per shard, merged per query by global row (`merge_range_results`).
+        numpy in -> numpy out; torch CUDA tensor in -> CUDA tensors on the first device."""
+        torch = self._torch
+        is_t = type(queries).__module__.startswith("torch")
+        if is_t:
+            queries = queries.contiguous()
+            torch.cuda.current_stream(queries.device).synchronize()
+        jobs = [self._pool.submit(self._range_one, g, queries, radius, mode) for g in range(len(self.engines))]
+        res = [j.result() for j in jobs]
+        self._last_stats = [r[1] for r in res]
+        lims, D, I = merge_range_results([r[0] for r in res])
+        if is_t:
+            dev0 = torch.device("cuda", self.devices[0])
+            return (torch.from_numpy(lims).to(dev0), torch.from_numpy(D).to(dev0), torch.from_numpy(I).to(dev0))
+        return lims, D, I
 
     def download(self, src, dst: np.ndarray) -> None:
         """dst (host array) <- src (CUDA tensor on any of this engine's devices)."""

@@ -28,6 +28,7 @@
 #include "../../include/b2ip.h"
 #include "coarse_kernel.cuh"
 #include "select_kernels.cuh"
+#include "range_kernels.cuh"
 
 using namespace b2ip;
 
@@ -102,6 +103,12 @@ struct b2ip_index_s {
     DevBuf q16, eps2, thr, cnt, kept, flags, cand, qstage, qhalf, out_s, out_r, exact_scores, exact_misc,
         qlist, stage, seg_tab, gmax;
     int n_seg = 0;                        // row segments (b2ip_set_row_segments); 0 = row_offset
+    // range search (b2ip_range_search): hit pool and its per-(slab, query) table, dense-path
+    // scratch, and the answer held for b2ip_range_fetch
+    DevBuf range_pool, range_tab_off, range_tab_cnt, range_stat, range_counts, range_offs, range_lims,
+        range_batches, range_s, range_r;
+    int64_t range_total = 0;
+    bool range_held = false;
     std::vector<cudaEvent_t> ev_pool, ev_fin;
     cudaEvent_t ev_t0 = nullptr, ev_t1 = nullptr;
     b2ip_stats_t stats;
@@ -1199,6 +1206,349 @@ int search_device(b2ip_handle h, int64_t nq, const float* dq, int k, float* d_sc
     return B2IP_OK;
 }
 
+// ------------------------------------------------------------------------- range search
+// DESIGN 4.1f.  The hits of one call accumulate in range_pool.  Table entry (slab j, query slot i)
+// of a query batch (range_tab_off / range_tab_cnt) says where that query's hits in that slab are,
+// in ascending row order; range_gather_kernel concatenates them slab by slab.
+
+// grows b to at least `bytes`, keeping its first `used` bytes (the range search's own buffers:
+// no CUDA graph holds them, so ws_gen stays)
+int grow_keep(b2ip_handle h, DevBuf& b, size_t used, size_t bytes) {
+    if (b.bytes >= bytes) return B2IP_OK;
+    size_t want = std::max(bytes, b.bytes + b.bytes / 2);
+    void* p = nullptr;
+    cudaError_t e = cudaMalloc(&p, want);
+    if (e != cudaSuccess) { cudaGetLastError(); want = bytes; e = cudaMalloc(&p, want); }
+    if (e != cudaSuccess) {
+        cudaGetLastError();
+        return fail(h, B2IP_ERR_OOM, "cudaMalloc(%zu bytes) failed: %s", bytes, cudaGetErrorString(e));
+    }
+    if (used > 0) {
+        e = cudaMemcpyAsync(p, b.p, used, cudaMemcpyDeviceToDevice, h->stream);
+        if (e == cudaSuccess) e = cudaStreamSynchronize(h->stream);
+        if (e != cudaSuccess) { cudaFree(p); CU_TRY(h, e); }
+    }
+    release(b);
+    b.p = p;
+    b.bytes = want;
+    return B2IP_OK;
+}
+
+struct RangeRun {
+    float radius;
+    int64_t qb = 0;                       // queries per batch
+    std::vector<long long> batches;       // per batch: first query, queries, slabs, first table entry
+    int64_t tab_used = 0;                 // table entries written
+    long long cursor = 0;                 // pool entries in use
+    std::vector<char> fell;               // queries that took the dense path for some slab
+    float drain_ms = 0.f, coarse_ms = 0.f;
+};
+
+int range_read_stat(b2ip_handle h, long long* rs) {
+    CU_TRY(h, cudaMemcpyAsync(rs, h->range_stat.p, RS_COUNT * sizeof(long long), cudaMemcpyDeviceToHost, h->stream));
+    CU_TRY(h, cudaStreamSynchronize(h->stream));
+    CU_TRY(h, cudaGetLastError());
+    return B2IP_OK;
+}
+
+template <bool kWrite>
+void launch_range_dense(b2ip_handle h, int grid, size_t smem, const RangeDenseParams& dp) {
+    if (h->x32) range_dense_kernel<ROWS_F32, kWrite><<<grid, 256, smem, h->stream>>>(dp);
+    else if (h->sh == SH_F16) range_dense_kernel<ROWS_F16, kWrite><<<grid, 256, smem, h->stream>>>(dp);
+    else range_dense_kernel<ROWS_BF16, kWrite><<<grid, 256, smem, h->stream>>>(dp);
+}
+
+// Exact hits of the queries `slots` (indices into q32) among rows [row0, row1): count per tile,
+// reserve each query one run of the pool, write.  Sets table entries tab_base + slot.
+int range_dense(b2ip_handle h, RangeRun& run, const float* q32, const std::vector<int>& slots,
+                int64_t row0, int64_t row1, int64_t tab_base) {
+    const int64_t ntiles = (row1 - row0 + RANGE_TILE - 1) / RANGE_TILE;
+    if (ntiles <= 0 || slots.empty()) return B2IP_OK;
+    // queries per round: the per-(query, tile) counts and positions stay within ~256 MiB
+    int64_t per = std::max<int64_t>(EXACT_QB, (256ll << 20) / (ntiles * 12) / EXACT_QB * EXACT_QB);
+    per = std::min<int64_t>(per, static_cast<int64_t>(slots.size()));
+    const bool rows16 = h->x32 == nullptr;
+    RangeDenseParams dp{};
+    dp.d = h->d;
+    dp.row_bytes = rows16 ? static_cast<long long>(h->d_pad) * 2 : static_cast<long long>(h->d) * 4;
+    dp.n_chunks = static_cast<int>(dp.row_bytes / 16);
+    dp.rows = rows16 ? reinterpret_cast<const char*>(h->x16) : reinterpret_cast<const char*>(h->x32);
+    dp.q32 = q32;
+    dp.row0 = row0;
+    dp.row1 = row1;
+    dp.ntiles = static_cast<int>(ntiles);
+    dp.radius = run.radius;
+    const size_t smem = static_cast<size_t>(EXACT_QB) * h->d * sizeof(float);
+    for (size_t s0 = 0; s0 < slots.size(); s0 += static_cast<size_t>(per)) {
+        const int nr = static_cast<int>(std::min<int64_t>(per, static_cast<int64_t>(slots.size() - s0)));
+        RC_TRY(grow_keep(h, h->qlist, 0, static_cast<size_t>(nr) * sizeof(int)));
+        RC_TRY(grow_keep(h, h->range_counts, 0, static_cast<size_t>(nr) * ntiles * sizeof(int)));
+        RC_TRY(grow_keep(h, h->range_offs, 0, static_cast<size_t>(nr) * ntiles * sizeof(long long)));
+        CU_TRY(h, cudaMemcpyAsync(h->qlist.p, slots.data() + s0, static_cast<size_t>(nr) * sizeof(int),
+                                  cudaMemcpyHostToDevice, h->stream));
+        dp.qlist = static_cast<const int*>(h->qlist.p);
+        dp.nql = nr;
+        dp.n_groups = (nr + EXACT_QB - 1) / EXACT_QB;
+        dp.counts = static_cast<int*>(h->range_counts.p);
+        dp.offs = static_cast<const long long*>(h->range_offs.p);
+        const int64_t gx = std::max<int64_t>(1, std::min<int64_t>(ntiles, (static_cast<int64_t>(h->sm_count) * 8 + dp.n_groups - 1) / dp.n_groups));
+        const int grid = static_cast<int>(gx * dp.n_groups);
+        const long long used = run.cursor;
+        launch_range_dense<false>(h, grid, smem, dp);
+        range_scan_kernel<<<nr, 256, 0, h->stream>>>(static_cast<const int*>(h->range_counts.p),
+                                                     static_cast<long long*>(h->range_offs.p), dp.ntiles,
+                                                     dp.qlist, static_cast<long long*>(h->range_tab_off.p) + tab_base,
+                                                     static_cast<int*>(h->range_tab_cnt.p) + tab_base,
+                                                     static_cast<long long*>(h->range_stat.p));
+        long long rs[RS_COUNT];
+        RC_TRY(range_read_stat(h, rs));
+        run.cursor = rs[RS_CURSOR];
+        RC_TRY(grow_keep(h, h->range_pool, static_cast<size_t>(used) * 8, static_cast<size_t>(std::max(run.cursor, 1ll)) * 8));
+        dp.pool = static_cast<unsigned long long*>(h->range_pool.p);
+        launch_range_dense<true>(h, grid, smem, dp);
+        CU_TRY(h, cudaGetLastError());
+        h->stats.total_launches += 3;
+    }
+    return B2IP_OK;
+}
+
+// Coarse pass with the fixed threshold rd(radius - eps_q), slab by slab; every slab is drained.
+int range_tensor(b2ip_handle h, RangeRun& run, const float* q32, int64_t nq) {
+    const int64_t n = h->n;
+    const int cap = SORT_CAP;             // a drained list is sorted in shared memory
+    int64_t qb_max = h->cand_budget_bytes / (static_cast<int64_t>(cap) * 8);
+    qb_max = std::max<int64_t>(TILE_Q, qb_max / TILE_Q * TILE_Q);
+    const int64_t qb = std::min<int64_t>(nq, qb_max);
+    run.qb = qb;
+    RC_TRY(ensure(h, h->q16, static_cast<size_t>(pad_q(qb)) * h->d_pad * 2));
+    RC_TRY(ensure(h, h->eps2, qb * sizeof(float)));
+    RC_TRY(ensure(h, h->thr, qb * sizeof(float)));
+    RC_TRY(ensure(h, h->cnt, qb * sizeof(int)));
+    RC_TRY(ensure(h, h->kept, qb * sizeof(int)));
+    RC_TRY(ensure(h, h->flags, qb * sizeof(int)));
+    RC_TRY(ensure(h, h->cand, static_cast<size_t>(qb) * cap * 8));
+    if (h->tmap_x_base != h->x16 || h->tmap_x_rows != n) {
+        RC_TRY(make_tmap_bf16(h, &h->tmap_x_pair, h->x16, n, h->d_pad, 128));
+        RC_TRY(make_tmap_bf16(h, &h->tmap_x, h->x16, n, h->d_pad, TILE_X));
+        h->tmap_x_base = h->x16;
+        h->tmap_x_rows = n;
+    }
+    const bool rows16 = h->x32 == nullptr;
+    RangeDrainParams rp{};
+    rp.cap = cap;
+    rp.d = h->d;
+    rp.row_bytes = rows16 ? static_cast<long long>(h->d_pad) * 2 : static_cast<long long>(h->d) * 4;
+    rp.n_chunks = static_cast<int>(rp.row_bytes / 16);
+    rp.rows = rows16 ? reinterpret_cast<const char*>(h->x16) : reinterpret_cast<const char*>(h->x32);
+    rp.eps2 = static_cast<const float*>(h->eps2.p);
+    rp.cand = static_cast<unsigned long long*>(h->cand.p);
+    rp.cnt = static_cast<int*>(h->cnt.p);
+    rp.flags = static_cast<int*>(h->flags.p);
+    rp.radius = run.radius;
+    rp.rstat = static_cast<long long*>(h->range_stat.p);
+    rp.gstats = h->gstats;
+    const size_t drain_smem = static_cast<size_t>(cap) * 8 + static_cast<size_t>(h->d) * 4;
+    cudaEvent_t e0 = get_event(h, 0), e1 = get_event(h, 1), e2 = get_event(h, 2);
+    long long rs[RS_COUNT];
+
+    for (int64_t q0 = 0; q0 < nq; q0 += qb) {
+        const int nqb = static_cast<int>(std::min<int64_t>(qb, nq - q0));
+        const float* qptr = q32 + q0 * h->d;
+        const int nq_pad = static_cast<int>(pad_q(nqb));
+        const size_t bi = run.batches.size();
+        run.batches.insert(run.batches.end(), {static_cast<long long>(q0), nqb, 0, static_cast<long long>(run.tab_used)});
+        h->stats.query_batches++;
+        CUtensorMap tmap_q;
+        RC_TRY(make_tmap_bf16(h, &tmap_q, h->q16.p, nq_pad, h->d_pad, TILE_Q));
+        const bool use_pair = h->pair && nqb > TILE_Q && h->sm_count >= 2;
+        prep_queries_kernel<<<(nq_pad + 7) / 8, 256, 0, h->stream>>>(
+            qptr, reinterpret_cast<__nv_bfloat16*>(h->q16.p), nqb, h->d, h->d_pad, h->norm_stats,
+            reinterpret_cast<float*>(h->eps2.p), reinterpret_cast<float*>(h->thr.p),
+            reinterpret_cast<int*>(h->cnt.p), reinterpret_cast<int*>(h->kept.p),
+            reinterpret_cast<int*>(h->flags.p), h->sh, nq_pad, h->gstats, 0, nullptr);
+        range_threshold_kernel<<<(nqb + 255) / 256, 256, 0, h->stream>>>(
+            static_cast<const float*>(h->eps2.p), static_cast<float*>(h->thr.p), nqb, run.radius);
+        h->stats.total_launches += 2;
+        rp.q32 = qptr;
+
+        CoarseParams cp{};
+        cp.num_k_blocks = h->d_pad / KBLOCK_ELEMS;
+        cp.q_tiles = use_pair ? (nqb + 2 * TILE_Q - 1) / (2 * TILE_Q) : (nqb + TILE_Q - 1) / TILE_Q;
+        cp.gx = h->gx;
+        cp.nq = nqb;
+        cp.thr = reinterpret_cast<float*>(h->thr.p);
+        cp.cand = rp.cand;
+        cp.cnt = rp.cnt;
+        cp.cap = cap;
+        cp.hint_q = hint_policy(h->hint_q);
+        cp.hint_x = hint_policy(h->hint_x);
+        cp.idesc = use_pair ? IDESC_PAIR[h->sh] : IDESC_SINGLE[h->sh];
+        cp.dense = 0;
+
+        // The first slab holds cap rows, so its lists cannot overflow.  Later slabs are sized from
+        // the largest admission rate per row seen so far: expected fill list_fill_pct % of cap.
+        int64_t done = 0, slab = cap;
+        double rate = 0.0;
+        while (done < n) {
+            int64_t s = std::min<int64_t>(slab, n - done);
+            s = std::min<int64_t>(s, std::max<int64_t>(1, (1ll << 30) / std::max(1, cp.q_tiles)) * STREAM_TILE_X);
+            if (done + s < n) s = std::max<int64_t>(TILE_X, s / TILE_X * TILE_X);
+            s = std::min<int64_t>(s, n - done);
+            const int64_t tab = run.tab_used;
+            RC_TRY(grow_keep(h, h->range_tab_off, static_cast<size_t>(tab) * 8, static_cast<size_t>(tab + nqb) * 8));
+            RC_TRY(grow_keep(h, h->range_tab_cnt, static_cast<size_t>(tab) * 4, static_cast<size_t>(tab + nqb) * 4));
+            RC_TRY(grow_keep(h, h->range_pool, static_cast<size_t>(run.cursor) * 8,
+                             static_cast<size_t>(run.cursor + static_cast<int64_t>(nqb) * std::min<int64_t>(cap, s)) * 8));
+            rp.pool = static_cast<unsigned long long*>(h->range_pool.p);
+            rp.tab_off = static_cast<long long*>(h->range_tab_off.p) + tab;
+            rp.tab_cnt = static_cast<int*>(h->range_tab_cnt.p) + tab;
+            CU_TRY(h, cudaMemsetAsync(static_cast<long long*>(h->range_stat.p) + RS_MAX_CNT, 0,
+                                      (RS_COUNT - RS_MAX_CNT) * sizeof(long long), h->stream));
+            cp.x_row0 = done;
+            cp.x_row_end = done + s;
+            cp.x_tiles = static_cast<int>((s + TILE_X - 1) / TILE_X);
+            const long long tiles = static_cast<long long>(cp.q_tiles) * cp.x_tiles;
+            CU_TRY(h, cudaEventRecord(e0, h->stream));
+            if (use_pair) {
+                const int grid = 2 * static_cast<int>(std::min<long long>(tiles, h->sm_count / 2));
+                coarse_filter_pair_kernel<<<grid, COARSE_THREADS, PAIR_SMEM_BYTES, h->stream>>>(
+                    tmap_q, h->tmap_x_pair, cp);
+            } else {
+                const int grid = static_cast<int>(std::min<long long>(tiles, h->sm_count));
+                coarse_filter_kernel<false><<<grid, COARSE_THREADS, COARSE_SMEM_BYTES, h->stream>>>(
+                    tmap_q, h->tmap_x, cp);
+            }
+            CU_TRY(h, cudaEventRecord(e1, h->stream));
+            if (!rows16) range_drain_kernel<ROWS_F32><<<nqb, SEL_THREADS, drain_smem, h->stream>>>(rp);
+            else if (h->sh == SH_F16) range_drain_kernel<ROWS_F16><<<nqb, SEL_THREADS, drain_smem, h->stream>>>(rp);
+            else range_drain_kernel<ROWS_BF16><<<nqb, SEL_THREADS, drain_smem, h->stream>>>(rp);
+            CU_TRY(h, cudaEventRecord(e2, h->stream));
+            CU_TRY(h, cudaMemcpyAsync(h->h_gstats, h->gstats, GS_COUNT * sizeof(long long),
+                                      cudaMemcpyDeviceToHost, h->stream));
+            RC_TRY(range_read_stat(h, rs));
+            float ms = 0.f;
+            if (cudaEventElapsedTime(&ms, e0, e1) == cudaSuccess) run.coarse_ms += ms;
+            if (cudaEventElapsedTime(&ms, e1, e2) == cudaSuccess) run.drain_ms += ms;
+            cudaGetLastError();
+            run.cursor = rs[RS_CURSOR];
+            h->stats.coarse_launches++;
+            h->stats.total_launches += 2;
+            h->stats.slabs++;
+            h->stats.coarse_flops += 2.0 * nqb * static_cast<double>(s) * h->d;
+            if (rs[RS_OVERFLOW] > 0) {            // these (query, slab) pairs are scored densely
+                std::vector<int> hflags(nqb), slots;
+                CU_TRY(h, cudaMemcpyAsync(hflags.data(), h->flags.p, nqb * sizeof(int), cudaMemcpyDeviceToHost, h->stream));
+                CU_TRY(h, cudaStreamSynchronize(h->stream));
+                for (int i = 0; i < nqb; i++)
+                    if (hflags[i] & FLAG_OVERFLOW) { slots.push_back(i); run.fell[q0 + i] = 1; }
+                RC_TRY(range_dense(h, run, qptr, slots, done, done + s, tab));
+            }
+            run.tab_used += nqb;
+            run.batches[bi + 2]++;
+            done += s;
+            rate = std::max(rate, static_cast<double>(std::max<long long>(rs[RS_MAX_CNT], 1)) / static_cast<double>(s));
+            const double next = std::min(0.01 * h->list_fill_pct * cap / rate, 4.0e9);
+            slab = std::max<int64_t>(TILE_X, static_cast<int64_t>(next));
+        }
+        h->stats.candidates += h->h_gstats[GS_CANDIDATES];
+        h->stats.rescored += h->h_gstats[GS_RESCORED];
+        const unsigned int bits = static_cast<unsigned int>(h->h_gstats[GS_MAX_ERR]);
+        float r;
+        memcpy(&r, &bits, sizeof(r));
+        h->stats.max_err_over_eps = std::max(h->stats.max_err_over_eps, static_cast<double>(r));
+        h->stats.bound_violations += h->h_gstats[GS_VIOLATIONS];
+    }
+    return B2IP_OK;
+}
+
+// The whole range search of nq device queries; out_lims (host) [nq + 1].  The answer stays in
+// range_s / range_r for b2ip_range_fetch.
+int range_device(b2ip_handle h, int64_t nq, const float* dq, float radius, int mode, int64_t* out_lims) {
+    memset(&h->stats, 0, sizeof(h->stats));
+    h->timing_pending = false;
+    h->stats.nq = nq; h->stats.ntotal = h->n; h->stats.k = 0;
+    out_lims[0] = 0;
+    if (nq == 0 || h->n == 0) {
+        for (int64_t i = 0; i <= nq; i++) out_lims[i] = 0;
+        h->stats.mode_used = h->n == 0 ? B2IP_MODE_EXACT : (mode == B2IP_MODE_EXACT ? B2IP_MODE_EXACT : B2IP_MODE_TENSOR);
+        h->range_total = 0;
+        h->range_held = true;
+        return B2IP_OK;
+    }
+    CU_TRY(h, cudaEventRecord(h->ev_t0, h->stream));
+    RC_TRY(grow_keep(h, h->range_stat, 0, RS_COUNT * sizeof(long long)));
+    CU_TRY(h, cudaMemsetAsync(h->range_stat.p, 0, RS_COUNT * sizeof(long long), h->stream));
+    RangeRun run;
+    run.radius = radius;
+    run.fell.assign(static_cast<size_t>(nq), 0);
+    if (mode == B2IP_MODE_EXACT) {
+        h->stats.mode_used = B2IP_MODE_EXACT;
+        run.qb = nq;
+        run.batches = {0, static_cast<long long>(nq), 1, 0};
+        RC_TRY(grow_keep(h, h->range_tab_off, 0, static_cast<size_t>(nq) * 8));
+        RC_TRY(grow_keep(h, h->range_tab_cnt, 0, static_cast<size_t>(nq) * 4));
+        std::vector<int> all(static_cast<size_t>(nq));
+        for (int64_t i = 0; i < nq; i++) all[i] = static_cast<int>(i);
+        RC_TRY(range_dense(h, run, dq, all, 0, h->n, 0));
+        run.tab_used = nq;
+    } else {
+        h->stats.mode_used = B2IP_MODE_TENSOR;
+        RC_TRY(range_tensor(h, run, dq, nq));
+        for (char f : run.fell) h->stats.fallback_queries += f;
+    }
+    // CSR offsets on the host, then one gather in query order
+    std::vector<int> tab(static_cast<size_t>(run.tab_used));
+    CU_TRY(h, cudaMemcpyAsync(tab.data(), h->range_tab_cnt.p, tab.size() * sizeof(int), cudaMemcpyDeviceToHost, h->stream));
+    CU_TRY(h, cudaStreamSynchronize(h->stream));
+    for (int64_t i = 0; i <= nq; i++) out_lims[i] = 0;
+    for (size_t b = 0; b < run.batches.size(); b += 4) {
+        const long long q0 = run.batches[b], nqb = run.batches[b + 1], slabs = run.batches[b + 2], first = run.batches[b + 3];
+        for (long long j = 0; j < slabs; j++)
+            for (long long i = 0; i < nqb; i++) out_lims[q0 + i + 1] += tab[first + j * nqb + i];
+    }
+    for (int64_t i = 0; i < nq; i++) out_lims[i + 1] += out_lims[i];
+    const int64_t total = out_lims[nq];
+    cudaEvent_t g0 = get_event(h, 0);
+    CU_TRY(h, cudaEventRecord(g0, h->stream));
+    if (total > 0) {
+        RC_TRY(grow_keep(h, h->range_s, 0, static_cast<size_t>(total) * sizeof(float)));
+        RC_TRY(grow_keep(h, h->range_r, 0, static_cast<size_t>(total) * sizeof(int64_t)));
+        RC_TRY(grow_keep(h, h->range_lims, 0, static_cast<size_t>(nq + 1) * sizeof(int64_t)));
+        RC_TRY(grow_keep(h, h->range_batches, 0, run.batches.size() * sizeof(long long)));
+        CU_TRY(h, cudaMemcpyAsync(h->range_lims.p, out_lims, static_cast<size_t>(nq + 1) * sizeof(int64_t),
+                                  cudaMemcpyHostToDevice, h->stream));
+        CU_TRY(h, cudaMemcpyAsync(h->range_batches.p, run.batches.data(), run.batches.size() * sizeof(long long),
+                                  cudaMemcpyHostToDevice, h->stream));
+        range_gather_kernel<<<static_cast<unsigned int>(nq), 256, 0, h->stream>>>(
+            static_cast<const unsigned long long*>(h->range_pool.p), static_cast<const long long*>(h->range_tab_off.p),
+            static_cast<const int*>(h->range_tab_cnt.p), static_cast<const long long*>(h->range_lims.p),
+            static_cast<const long long*>(h->range_batches.p), run.qb, h->row_offset, h->n_seg,
+            static_cast<const long long*>(h->seg_tab.p), static_cast<const long long*>(h->seg_tab.p) + h->n_seg,
+            static_cast<float*>(h->range_s.p), static_cast<long long*>(h->range_r.p));
+        h->stats.total_launches++;
+    }
+    CU_TRY(h, cudaEventRecord(h->ev_t1, h->stream));
+    CU_TRY(h, cudaStreamSynchronize(h->stream));
+    CU_TRY(h, cudaGetLastError());
+    float ms = 0.f;
+    if (cudaEventElapsedTime(&ms, h->ev_t0, h->ev_t1) == cudaSuccess) h->stats.total_ms = ms;
+    if (cudaEventElapsedTime(&ms, g0, h->ev_t1) == cudaSuccess) run.drain_ms += ms;
+    cudaGetLastError();
+    h->stats.coarse_ms = run.coarse_ms;
+    h->stats.finalize_ms = run.drain_ms;
+    h->range_total = total;
+    h->range_held = true;
+    return B2IP_OK;
+}
+
+void range_release(b2ip_handle h) {
+    for (DevBuf* b : {&h->range_pool, &h->range_tab_off, &h->range_tab_cnt, &h->range_stat, &h->range_counts,
+                      &h->range_offs, &h->range_lims, &h->range_batches, &h->range_s, &h->range_r})
+        release(*b);
+    h->range_total = 0;
+    h->range_held = false;
+}
+
 }  // namespace
 
 // =========================================================================== C ABI
@@ -1288,6 +1638,18 @@ int b2ip_create_ex(int d, int device, int store_dtype, b2ip_handle* out) {
             cudaFuncSetAttribute(exact_scores_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                  static_cast<int>(static_cast<size_t>(EXACT_QB) * B2IP_MAX_D * sizeof(float))) != cudaSuccess)
             return bail(B2IP_ERR_CUDA, "cudaFuncSetAttribute(MaxDynamicSharedMemorySize)");
+        const int drain_smem = SORT_CAP * 8 + B2IP_MAX_D * 4;
+        const int dense_smem = EXACT_QB * B2IP_MAX_D * 4;
+        if (cudaFuncSetAttribute(range_drain_kernel<ROWS_F32>, cudaFuncAttributeMaxDynamicSharedMemorySize, drain_smem) != cudaSuccess ||
+            cudaFuncSetAttribute(range_drain_kernel<ROWS_BF16>, cudaFuncAttributeMaxDynamicSharedMemorySize, drain_smem) != cudaSuccess ||
+            cudaFuncSetAttribute(range_drain_kernel<ROWS_F16>, cudaFuncAttributeMaxDynamicSharedMemorySize, drain_smem) != cudaSuccess ||
+            cudaFuncSetAttribute(range_dense_kernel<ROWS_F32, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, dense_smem) != cudaSuccess ||
+            cudaFuncSetAttribute(range_dense_kernel<ROWS_BF16, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, dense_smem) != cudaSuccess ||
+            cudaFuncSetAttribute(range_dense_kernel<ROWS_F16, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, dense_smem) != cudaSuccess ||
+            cudaFuncSetAttribute(range_dense_kernel<ROWS_F32, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, dense_smem) != cudaSuccess ||
+            cudaFuncSetAttribute(range_dense_kernel<ROWS_BF16, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, dense_smem) != cudaSuccess ||
+            cudaFuncSetAttribute(range_dense_kernel<ROWS_F16, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, dense_smem) != cudaSuccess)
+            return bail(B2IP_ERR_CUDA, "cudaFuncSetAttribute(MaxDynamicSharedMemorySize)");
     }
     h->gx = std::max(1, h->sm_count / 2);   // = clusters of the pair kernel: one query tile per wave,
                                             // the corpus tiles of a group stay L2 resident (measured best)
@@ -1313,6 +1675,7 @@ void b2ip_destroy(b2ip_handle h) {
                       &h->out_s, &h->out_r, &h->exact_scores, &h->exact_misc, &h->qlist, &h->stage,
                       &h->seg_tab, &h->gmax})
         release(*b);
+    range_release(h);
     if (h->v16.base || h->v32.base) {
         vmm_free(h, h->v32);
         vmm_free(h, h->v16);
@@ -1400,6 +1763,10 @@ int b2ip_add(b2ip_handle h, int64_t n, const void* rows, int src_dtype, int mem)
     // rows handed in in the storage type itself are copied as they are
     const bool same16 = h->store16 && ((src_dtype == B2IP_BF16 && h->sh == SH_BF16) ||
                                        (src_dtype == B2IP_F16 && h->sh == SH_F16));
+    {   // the held range search answer no longer describes the index
+        Guard g(h->device);
+        range_release(h);
+    }
     if (n == 0) return B2IP_OK;
     if (h->n + n >= (1ll << 31) - 512) return fail(h, B2IP_ERR_UNSUPPORTED, "a shard holds at most 2^31-512 rows (TMA coordinates are int32)");
     Guard g(h->device);
@@ -1623,6 +1990,66 @@ int b2ip_search_exchange(b2ip_handle h, int64_t nq, const float* queries_dev, in
                     "(B2IP_EXCHANGE_TIMEOUT_S): the peer is gone or stuck; this rank's view of the "
                     "exchange is no longer consistent with its peers -- tear the process group down",
                     seq, h->ex_timeout_ns * 1e-9);
+    return B2IP_OK;
+}
+
+int b2ip_range_search(b2ip_handle h, int64_t nq, const void* queries, int q_dtype, float radius,
+                      int mode, int mem, int64_t* out_lims) {
+    if (!h) return B2IP_ERR_INVALID;
+    if (h->d <= 0) return fail(h, B2IP_ERR_INVALID, "b2ip_range_search: the index has no dimension");
+    if (q_dtype != B2IP_F32 && q_dtype != B2IP_F16)
+        return fail(h, B2IP_ERR_INVALID, "b2ip_range_search: q_dtype=%d (use B2IP_F32 or B2IP_F16)", q_dtype);
+    if (nq < 0 || !out_lims || (nq > 0 && !queries))
+        return fail(h, B2IP_ERR_INVALID, "b2ip_range_search: NULL buffer or nq=%lld", (long long)nq);
+    if (mode < B2IP_MODE_AUTO || mode > B2IP_MODE_EXACT) return fail(h, B2IP_ERR_INVALID, "b2ip_range_search: mode=%d", mode);
+    if (mem != B2IP_MEM_HOST && mem != B2IP_MEM_DEVICE) return fail(h, B2IP_ERR_INVALID, "b2ip_range_search: mem=%d", mem);
+    if (radius != radius) return fail(h, B2IP_ERR_INVALID, "b2ip_range_search: radius is NaN");
+    if (nq >= (1ll << 31)) return fail(h, B2IP_ERR_UNSUPPORTED, "b2ip_range_search: nq too large");
+    if (h->n_seg == 0 && h->row_offset + h->n > MAX_GLOBAL_ROWS)
+        return fail(h, B2IP_ERR_UNSUPPORTED, "b2ip_range_search: row offset %lld + %lld rows exceeds 2^32 - 1 global row ids",
+                    (long long)h->row_offset, (long long)h->n);
+    Guard g(h->device);
+    h->range_held = false;
+    const float* dq = static_cast<const float*>(queries);
+    if (nq > 0 && h->n > 0 && (mem == B2IP_MEM_HOST || q_dtype == B2IP_F16)) {
+        // fp32 queries on the device as b2ip_search_ex stages them (float16 widened exactly)
+        const size_t q_count = static_cast<size_t>(nq) * h->d;
+        RC_TRY(ensure(h, h->qstage, q_count * sizeof(float)));
+        const void* half_dev = queries;
+        if (mem == B2IP_MEM_HOST && q_dtype == B2IP_F16) {
+            RC_TRY(ensure(h, h->qhalf, q_count * 2));
+            RC_TRY(host_to_device(h, h->qhalf.p, queries, q_count * 2));
+            half_dev = h->qhalf.p;
+        } else if (mem == B2IP_MEM_HOST) {
+            RC_TRY(host_to_device(h, h->qstage.p, queries, q_count * sizeof(float)));
+        }
+        if (q_dtype == B2IP_F16) {
+            const int grid = static_cast<int>(std::min<size_t>((q_count / 2 + 255) / 256 + 1, 65535));
+            widen_f16_kernel<<<grid, 256, 0, h->stream>>>(static_cast<const __half*>(half_dev),
+                                                          static_cast<float*>(h->qstage.p),
+                                                          static_cast<long long>(q_count));
+        }
+        dq = static_cast<const float*>(h->qstage.p);
+    }
+    return range_device(h, nq, dq, radius, mode, out_lims);
+}
+
+int b2ip_range_fetch(b2ip_handle h, float* out_scores, int64_t* out_rows, int mem) {
+    if (!h) return B2IP_ERR_INVALID;
+    if (!h->range_held) return fail(h, B2IP_ERR_INVALID, "b2ip_range_fetch: no range search answer is held");
+    if (mem != B2IP_MEM_HOST && mem != B2IP_MEM_DEVICE) return fail(h, B2IP_ERR_INVALID, "b2ip_range_fetch: mem=%d", mem);
+    const int64_t total = h->range_total;
+    if (total == 0) return B2IP_OK;
+    if (!out_scores || !out_rows) return fail(h, B2IP_ERR_INVALID, "b2ip_range_fetch: NULL buffer");
+    Guard g(h->device);
+    const size_t sb = static_cast<size_t>(total) * sizeof(float), rb = static_cast<size_t>(total) * sizeof(int64_t);
+    if (mem == B2IP_MEM_HOST) {
+        RC_TRY(device_to_host(h, out_scores, h->range_s.p, sb));
+        return device_to_host(h, out_rows, h->range_r.p, rb);
+    }
+    CU_TRY(h, cudaMemcpyAsync(out_scores, h->range_s.p, sb, cudaMemcpyDeviceToDevice, h->stream));
+    CU_TRY(h, cudaMemcpyAsync(out_rows, h->range_r.p, rb, cudaMemcpyDeviceToDevice, h->stream));
+    CU_TRY(h, cudaStreamSynchronize(h->stream));
     return B2IP_OK;
 }
 

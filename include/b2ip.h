@@ -157,6 +157,26 @@ int b2ip_search(b2ip_handle h, int64_t nq, const float* queries, int k, float* o
 int b2ip_search_ex(b2ip_handle h, int64_t nq, const void* queries, int q_dtype, int k,
                    float* out_scores, int64_t* out_rows, int mode, int mem);
 
+/* replaces lims, D, I = index.range_search(q, radius) (faiss IndexFlatIP).
+ * queries [nq,d] fp32 or fp16 (q_dtype), mode B2IP_MODE_AUTO/TENSOR/EXACT.  Computes the answer,
+ * keeps it in library memory and writes the host array out_lims[nq+1] (out_lims[nq] = total).
+ * Query i's results are entries [out_lims[i], out_lims[i+1]) of the answer: every row whose exact
+ * score s satisfies s > radius (strict, as faiss; NaN never), in ascending row order, ids mapped
+ * as b2ip_search maps them.  s is computed by the same arithmetic as b2ip_search's rescore, so a
+ * row both return gets bit-identical scores; TENSOR and EXACT give bit-identical answers.
+ * radius = -inf returns every row with a non-NaN score above -inf; a NaN radius is rejected.
+ * There is no result cap (memory grows as needed; B2IP_ERR_OOM leaves the handle usable).
+ * `mem` says where the queries live.  b2ip_stats afterwards: k = 0, candidates = pairs admitted
+ * by the coarse pass, rescored, fallback_queries = queries scored densely for some slab,
+ * finalize_ms = drain + gather kernels, and the certificate max_err_over_eps / bound_violations. */
+int b2ip_range_search(b2ip_handle h, int64_t nq, const void* queries, int q_dtype, float radius,
+                      int mode, int mem, int64_t* out_lims);
+
+/* Copies the answer of the last b2ip_range_search on h: scores [total] fp32, rows [total] int64
+ * (mem = where the caller's buffers live).  B2IP_ERR_INVALID when no answer is held.  The held
+ * answer is released by the next b2ip_range_search, by b2ip_add and by b2ip_destroy. */
+int b2ip_range_fetch(b2ip_handle h, float* out_scores, int64_t* out_rows, int mem);
+
 /* The one exchange step of the row-sharded search: merges n_lists per-shard results
  * (scores [n_lists,nq,k] descending per list, rows [n_lists,nq,k] global ids, -1 padded)
  * into the global top-k (score desc, ties -> lower row).  All pointers are DEVICE
