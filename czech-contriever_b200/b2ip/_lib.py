@@ -21,7 +21,7 @@ MAX_K = 2048
 # every symbol include/b2ip.h declares (tests check the .so exports all of them)
 SYMBOLS = (
     "b2ip_create", "b2ip_create_ex", "b2ip_destroy", "b2ip_set_stream", "b2ip_set_option", "b2ip_reserve", "b2ip_add", "b2ip_ntotal",
-    "b2ip_dim", "b2ip_set_row_offset", "b2ip_set_row_segments", "b2ip_search", "b2ip_search_ex", "b2ip_range_search", "b2ip_range_fetch", "b2ip_search_exchange", "b2ip_enable_peer_access", "b2ip_group_create", "b2ip_group_destroy", "b2ip_group_search", "b2ip_group_last_error",
+    "b2ip_dim", "b2ip_set_row_offset", "b2ip_set_row_segments", "b2ip_search", "b2ip_search_ex", "b2ip_search_filtered", "b2ip_range_search", "b2ip_range_fetch", "b2ip_search_exchange", "b2ip_enable_peer_access", "b2ip_group_create", "b2ip_group_destroy", "b2ip_group_search", "b2ip_group_last_error",
     "b2ip_merge_topk", "b2ip_merge_topk_strided", "b2ip_export_rows",
     "b2ip_copy_to_device", "b2ip_copy_to_host", "b2ip_stats", "b2ip_last_error", "b2ip_debug_coarse_scores", "b2ip_debug_plan_bootstrap", "b2ip_version",
 )
@@ -95,6 +95,7 @@ def load() -> ctypes.CDLL:
     lib.b2ip_set_row_segments.argtypes = [vp, i32, vp, vp]
     lib.b2ip_search.argtypes = [vp, i64, vp, i32, vp, vp, i32, i32]
     lib.b2ip_search_ex.argtypes = [vp, i64, vp, i32, i32, vp, vp, i32, i32]
+    lib.b2ip_search_filtered.argtypes = [vp, i64, vp, i32, i32, vp, i64, vp, vp, i32, i32]
     lib.b2ip_range_search.argtypes = [vp, i64, vp, i32, ctypes.c_float, i32, i32, vp]
     lib.b2ip_range_fetch.argtypes = [vp, vp, vp, i32]
     lib.b2ip_search_exchange.argtypes = [vp, i64, vp, i32, ctypes.POINTER(Exchange), ctypes.c_uint32, vp, vp,
@@ -122,7 +123,7 @@ def load() -> ctypes.CDLL:
     lib.b2ip_debug_plan_bootstrap.restype = i32
     lib.b2ip_version.restype = ctypes.c_char_p
     for name in ("b2ip_create", "b2ip_create_ex", "b2ip_set_stream", "b2ip_set_option", "b2ip_reserve", "b2ip_add", "b2ip_dim",
-                 "b2ip_set_row_offset", "b2ip_set_row_segments", "b2ip_search", "b2ip_search_ex", "b2ip_range_search", "b2ip_range_fetch", "b2ip_search_exchange", "b2ip_enable_peer_access", "b2ip_merge_topk", "b2ip_merge_topk_strided",
+                 "b2ip_set_row_offset", "b2ip_set_row_segments", "b2ip_search", "b2ip_search_ex", "b2ip_search_filtered", "b2ip_range_search", "b2ip_range_fetch", "b2ip_search_exchange", "b2ip_enable_peer_access", "b2ip_merge_topk", "b2ip_merge_topk_strided",
                  "b2ip_export_rows", "b2ip_stats", "b2ip_debug_coarse_scores", "b2ip_copy_to_device",
                  "b2ip_copy_to_host"):
         getattr(lib, name).restype = i32

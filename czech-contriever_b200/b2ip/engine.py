@@ -23,6 +23,27 @@ def _is_torch(x) -> bool:
     return type(x).__module__.startswith("torch")
 
 
+def pack_allowed(allowed):
+    """Allowed-row mask (bool, one entry per row) -> the bitmap b2ip_search_filtered reads: bit r & 31
+    of 32-bit word r >> 5 is set when row r may be returned.  This is np.packbits(mask,
+    bitorder="little") padded to whole words.  numpy in -> uint32 numpy array; torch tensor in ->
+    int32 tensor (the same bits) on the tensor's device."""
+    if _is_torch(allowed):
+        import torch
+        if allowed.dtype != torch.bool or allowed.dim() != 1:
+            raise ValueError("allowed must be a 1-d bool tensor")
+        n = allowed.shape[0]
+        m = torch.zeros(-(-n // 32) * 32, dtype=torch.uint8, device=allowed.device)
+        m[:n] = allowed
+        shifts = torch.arange(8, dtype=torch.uint8, device=allowed.device)
+        return (m.view(-1, 8) << shifts).sum(1, dtype=torch.uint8).view(torch.int32)
+    a = np.asarray(allowed)
+    if a.dtype != np.bool_ or a.ndim != 1:
+        raise ValueError("allowed must be a 1-d bool array")
+    b = np.packbits(a, bitorder="little")
+    return np.pad(b, (0, -len(b) % 4)).view("<u4")
+
+
 class Engine:
     def __init__(self, d: int, device: int = 0, store: str = "f32", shadow: Optional[str] = None):
         """store="f32": fp32 master rows (faiss semantics) + a 16-bit shadow for the coarse pass
@@ -136,9 +157,37 @@ class Engine:
         return out
 
     # -- search --------------------------------------------------------------------
-    def search(self, queries, k: int, mode: str = "auto", out=None) -> Tuple[object, object]:
+    def _search_call(self, nq, q_ptr, q_dtype, k, d_ptr, i_ptr, m, mem, allowed):
+        if allowed is None:
+            return self._lib.b2ip_search_ex(self._h, nq, q_ptr, q_dtype, k, d_ptr, i_ptr, m, mem)
+        if len(allowed) != self.ntotal:
+            raise ValueError(f"allowed has {len(allowed)} entries, the index holds {self.ntotal} rows")
+        if _is_torch(allowed) and allowed.is_cuda and allowed.device.index != self.device:
+            raise ValueError(f"allowed lives on {allowed.device}, the engine on cuda:{self.device}")
+        bits = pack_allowed(allowed)
+        # the bitmap crosses the ABI where the queries do (`mem`): wherever the mask was packed
+        # (host numpy, a CPU or a CUDA tensor), move it there
+        if mem == MEM_DEVICE:
+            import torch
+            if not _is_torch(bits):
+                bits = torch.from_numpy(bits.view(np.int32))
+            bits = bits.to(torch.device("cuda", self.device))
+            self._order_after_torch()          # packed / copied on torch's stream
+            ptr = bits.data_ptr()
+        else:
+            if _is_torch(bits):
+                bits = bits.cpu().numpy()
+            ptr = bits.ctypes.data
+        return self._lib.b2ip_search_filtered(self._h, nq, q_ptr, q_dtype, k, ctypes.c_void_p(ptr), len(allowed),
+                                              d_ptr, i_ptr, m, mem)
+
+    def search(self, queries, k: int, mode: str = "auto", out=None, allowed=None) -> Tuple[object, object]:
         """(scores [nq,k] float32 descending, rows [nq,k] int64).  numpy in -> numpy out (host
-        buffers cross the ABI, H2D/D2H inside the call); torch CUDA tensor in -> tensors out."""
+        buffers cross the ABI, H2D/D2H inside the call); torch CUDA tensor in -> tensors out.
+        `allowed` (bool, one entry per row: numpy, or a torch bool tensor on the engine's GPU)
+        restricts the search to the rows it marks (faiss SearchParameters(sel=IDSelectorBitmap)):
+        the answer is that of an index holding only those rows, with the original row ids; the
+        tail is (-FLT_MAX, -1) when fewer than k allowed rows have a score."""
         m = _MODES[mode]
         k = int(k)
         if _is_torch(queries):
@@ -155,10 +204,10 @@ class Engine:
             else:
                 D, I = out
             self._order_after_torch()
-            check(self._lib.b2ip_search_ex(self._h, nq, ctypes.c_void_p(q.data_ptr()),
-                                           B2IP_F16 if q.dtype == torch.float16 else B2IP_F32, k,
-                                           ctypes.c_void_p(D.data_ptr()), ctypes.c_void_p(I.data_ptr()),
-                                           m, MEM_DEVICE), self._h)
+            check(self._search_call(nq, ctypes.c_void_p(q.data_ptr()),
+                                    B2IP_F16 if q.dtype == torch.float16 else B2IP_F32, k,
+                                    ctypes.c_void_p(D.data_ptr()), ctypes.c_void_p(I.data_ptr()),
+                                    m, MEM_DEVICE, allowed), self._h)
             return D, I
         q = np.asarray(queries)
         if q.dtype not in (np.float16, np.float32):
@@ -172,10 +221,10 @@ class Engine:
             I = np.empty((nq, k), dtype=np.int64)
         else:
             D, I = out
-        check(self._lib.b2ip_search_ex(self._h, nq, ctypes.c_void_p(q.ctypes.data),
-                                       B2IP_F16 if q.dtype == np.float16 else B2IP_F32, k,
-                                       ctypes.c_void_p(D.ctypes.data), ctypes.c_void_p(I.ctypes.data),
-                                       m, MEM_HOST), self._h)
+        check(self._search_call(nq, ctypes.c_void_p(q.ctypes.data),
+                                B2IP_F16 if q.dtype == np.float16 else B2IP_F32, k,
+                                ctypes.c_void_p(D.ctypes.data), ctypes.c_void_p(I.ctypes.data),
+                                m, MEM_HOST, allowed), self._h)
         return D, I
 
     def range_search(self, queries, radius: float, mode: str = "auto"):

@@ -58,6 +58,7 @@ class Indexer(object):
         self.index = self._new_engine(vector_sz, "f16" if store == "f16" else "f32")
         self.index_id_to_db_id = []
         self.knn_chunk = 32768        # queries per pipelined search_knn chunk (env B2IP_KNN_CHUNK)
+        self._id_rows = None          # str(db_id) -> rows, built by the first filtered search_knn
 
     @classmethod
     def from_engine(cls, engine, ids=None, store=None) -> "Indexer":
@@ -69,6 +70,7 @@ class Indexer(object):
         self.index = engine
         self.index_id_to_db_id = list(ids) if ids is not None else []
         self.knn_chunk = 32768
+        self._id_rows = None
         return self
 
     def _new_engine(self, d, store):
@@ -96,6 +98,7 @@ class Indexer(object):
 
     def index_data(self, ids, embeddings):
         self._update_id_mapping(ids)
+        self._id_rows = None
         # reference: embeddings.astype('float32'); fp16 is widened on the GPU (exact)
         if self.store == "auto":
             if self._is_f16(embeddings):
@@ -108,7 +111,31 @@ class Indexer(object):
 
         print(f'Total data indexed {len(self.index_id_to_db_id)}')
 
-    def search_knn(self, query_vectors: np.array, top_docs: int, index_batch_size: int = 2048) -> List[Tuple[List[object], List[float]]]:
+    def allowed_mask(self, allowed_ids) -> np.ndarray:
+        """Bool mask over the indexed rows: True for every row whose external id, as `str`, is in
+        `allowed_ids` (duplicated ids: all their rows).  Unknown ids are ignored, as a faiss
+        selector ignores ids the index does not hold.  The id -> rows lookup is built on the first
+        call and kept until `index_data` or `deserialize_from` changes the ids."""
+        if self._id_rows is None:
+            first, dups = {}, {}
+            for r, s in enumerate(map(str, self.index_id_to_db_id)):
+                j = first.setdefault(s, r)
+                if j != r:
+                    dups.setdefault(s, [j]).append(r)
+            self._id_rows = (first, dups)
+        first, dups = self._id_rows
+        mask = np.zeros(len(self.index_id_to_db_id), dtype=bool)
+        rows = []
+        for a in set(map(str, allowed_ids)):
+            if a in dups:
+                rows.extend(dups[a])
+            elif a in first:
+                rows.append(first[a])
+        mask[np.asarray(rows, dtype=np.int64)] = True
+        return mask
+
+    def search_knn(self, query_vectors: np.array, top_docs: int, index_batch_size: int = 2048,
+                   allowed_ids=None) -> List[Tuple[List[object], List[float]]]:
         """reference src/index.py:34-46, same return value: nq tuples (list of k external ids as
         `str`, float32 score row), rows score-descending.  `query_vectors` may be a numpy array
         (float16 / float32 are handed to the library as they are -- float16 is widened on the
@@ -118,7 +145,11 @@ class Indexer(object):
 
         The queries are searched in chunks on a background thread while this thread maps the
         previous chunk's rows to external ids (csrc/hostmap.c: the reference's nq*k str() loop
-        in C), so the host half of the call hides behind the GPU half."""
+        in C), so the host half of the call hides behind the GPU half.
+
+        `allowed_ids` (an iterable of external ids, matched as `str`) restricts the search to
+        those passages (faiss SearchParameters(sel=...)); each tuple then holds only the real
+        results, fewer than `top_docs` when fewer passages are allowed, with no padding."""
         q = query_vectors
         on_device = False
         if _is_torch(q):
@@ -140,10 +171,14 @@ class Indexer(object):
         map_ids = load_hostmap().map_ids
         chunk = max(1, int(os.environ.get("B2IP_KNN_CHUNK", self.knn_chunk)))
         index = self.index
+        allowed = None if allowed_ids is None else self.allowed_mask(allowed_ids)
+        if allowed is not None and not ids:
+            return [([], np.empty(0, np.float32)) for _ in range(nq)]
 
         def searches():
             for s in range(0, nq, chunk):
-                D, I = index.search(q[s:s + chunk], top_docs)
+                D, I = index.search(q[s:s + chunk], top_docs) if allowed is None else \
+                    index.search(q[s:s + chunk], top_docs, allowed=allowed)
                 if on_device:
                     Dn = np.empty(tuple(D.shape), np.float32)
                     In = np.empty(tuple(I.shape), np.int64)
@@ -156,7 +191,12 @@ class Indexer(object):
         # convert to external ids (negative rows index from the end, like the reference's
         # `index_id_to_db_id[-1]` for faiss's -1 padding; an empty id list raises IndexError)
         for scores, indexes in prefetch(searches(), depth=2):
-            result.extend(map_ids(ids, indexes, indexes.shape[0], indexes.shape[1], list(scores)))
+            part = map_ids(ids, indexes, indexes.shape[0], indexes.shape[1], list(scores))
+            if allowed is not None:
+                # the -1 padding sits at the tail of a row: keep the real results only
+                n_real = (indexes >= 0).sum(axis=1).tolist()
+                part = [(i[:c], s[:c]) for (i, s), c in zip(part, n_real)]
+            result.extend(part)
         return result
 
     def search_range(self, query_vectors, radius: float) -> List[Tuple[List[object], np.ndarray]]:
@@ -211,6 +251,7 @@ class Indexer(object):
 
         with open(meta_file, "rb") as reader:
             self.index_id_to_db_id = pickle.load(reader)
+        self._id_rows = None
         assert len(
             self.index_id_to_db_id) == self.index.ntotal, 'Deserialized index_id_to_db_id should match faiss index size'
 

@@ -71,6 +71,16 @@ class SegmentMap:
         seg = torch.bucketize(rows_local.clamp(min=0), ls, right=True) - 1
         return torch.where(rows_local >= 0, rows_local + delta[seg], rows_local)
 
+    def local_mask(self, allowed):
+        """The shard's slice of a global allowed-row mask (numpy or torch bool, one entry per
+        global row), in local row order: the shard's segments are interleaved with the other
+        shards', so this is one slice per segment."""
+        parts = [allowed[gs:gs + n] for _, gs, n in self.segments]
+        if type(allowed).__module__.startswith("torch"):
+            import torch
+            return torch.cat(parts) if parts else allowed[:0]
+        return np.concatenate(parts) if parts else allowed[:0]
+
     def overlaps(self, g0: int, g1: int):
         """(local_start, global_start, n) pieces of this shard inside global rows [g0, g1)."""
         starts = [s[1] for s in self.segments]
@@ -204,12 +214,18 @@ class MultiGpuEngine:
         return out
 
     # -- search ----------------------------------------------------------------------
-    def _search_one(self, g: int, q_dev0, k: int, mode: str):
+    def _search_one(self, g: int, q_dev0, k: int, mode: str, allowed=None):
         torch = self._torch
         dev = torch.device("cuda", self.devices[g])
         with torch.cuda.device(dev):
             q = q_dev0 if q_dev0.device == dev else q_dev0.to(dev)      # fan-out over NVLink
-            D, I = self.engines[g].search(q, k, mode=mode)
+            if allowed is None:
+                D, I = self.engines[g].search(q, k, mode=mode)
+            else:
+                mask = self.maps[g].local_mask(allowed)
+                if type(mask).__module__.startswith("torch") and mask.device != dev:
+                    mask = mask.to(dev)
+                D, I = self.engines[g].search(q, k, mode=mode, allowed=mask)
             st = self.engines[g].stats()
             torch.cuda.current_stream(dev).synchronize()
         return D, I, st
@@ -308,8 +324,10 @@ class MultiGpuEngine:
                 self.engines[g].download(I, host_out[1][lo:hi])
         return D, I, st, status
 
-    def search(self, queries, k: int, mode: str = "auto", out=None):
-        """numpy in -> numpy out, torch CUDA tensor in -> tensors on the first device."""
+    def search(self, queries, k: int, mode: str = "auto", out=None, allowed=None):
+        """numpy in -> numpy out, torch CUDA tensor in -> tensors on the first device.  `allowed`
+        (bool per global row, numpy or torch) restricts the search as in `Engine.search`: each
+        shard searches its own slice of the mask and the per-shard results are merged."""
         torch = self._torch
         k = int(k)
         G = len(self.engines)
@@ -344,7 +362,10 @@ class MultiGpuEngine:
                         torch.empty((0, k), dtype=torch.int64, device=dev0))
             return host_out
         D = I = None
-        if not is_t and G > 1 and mode != "exact" and self._group_ok is not False:
+        if allowed is not None and len(allowed) != self._n:
+            raise ValueError(f"allowed has {len(allowed)} entries, the index holds {self._n} rows")
+        filtered = allowed is not None           # the fused exchange paths take no filter
+        if not is_t and G > 1 and mode != "exact" and self._group_ok is not False and not filtered:
             # host queries: ONE native call runs uploads, searches + fused exchange and downloads
             # of all GPUs on the library's own worker threads (b2ip_group_search)
             status = self._group_search(q_host, k, host_out)
@@ -354,7 +375,7 @@ class MultiGpuEngine:
                 return host_out
             if status is None:                       # no P2P path between the devices
                 pass
-        ex = self._exchange(nq, k) if (G > 1 and mode != "exact" and is_t) else None
+        ex = self._exchange(nq, k) if (G > 1 and mode != "exact" and is_t and not filtered) else None
         if ex is not None:
             self._x_seq += 1
             per = -(-nq // G)
@@ -370,7 +391,7 @@ class MultiGpuEngine:
                 with torch.cuda.device(dev0):
                     return (torch.cat([r[0].to(dev0) for r in res]), torch.cat([r[1].to(dev0) for r in res]))
             # a candidate list overflowed somewhere (same status on every device): repeat below
-        parts = [self._pool.submit(self._search_one, g, q_dev0, k, mode) for g in range(G)]
+        parts = [self._pool.submit(self._search_one, g, q_dev0, k, mode, allowed) for g in range(G)]
         res = [p.result() for p in parts]
         self._last_stats = [r[2] for r in res]
         with torch.cuda.device(dev0):

@@ -101,7 +101,7 @@ struct b2ip_index_s {
     PFN_encodeTiled encode = nullptr;
     // grow-only workspace
     DevBuf q16, eps2, thr, cnt, kept, flags, cand, qstage, qhalf, out_s, out_r, exact_scores, exact_misc,
-        qlist, stage, seg_tab, gmax;
+        qlist, stage, seg_tab, gmax, allow;
     int n_seg = 0;                        // row segments (b2ip_set_row_segments); 0 = row_offset
     // range search (b2ip_range_search): hit pool and its per-(slab, query) table, dense-path
     // scratch, and the answer held for b2ip_range_fetch
@@ -139,6 +139,8 @@ struct b2ip_index_s {
     int extra_rank[MAX_PEERS - 1] = {};     // rank that owns extra_base[e]
     bool ex_thr = false;                    // global threshold round active for this search
     long long ex_timeout_ns = 600ll * 1000000000ll;   // B2IP_EXCHANGE_TIMEOUT_S
+    // allowed-row bitmap of the current b2ip_search_filtered call (the `allow` buffer), nullptr otherwise
+    const uint32_t* filter = nullptr;
     // CUDA-graph replay of small-batch searches (fixed slab schedule): see tensor_search
     int graph = 1;                        // option "graph" / env B2IP_GRAPH
     int graph_timing = 0;                 // keep the per-kernel event records inside the graph (3 us per node:
@@ -150,6 +152,7 @@ struct b2ip_index_s {
     struct GraphEntry {
         int64_t nq, n; int k, cap;
         unsigned long long ws_gen, opt_gen;
+        bool filtered;                    // launches the _bitmap kernels (reads the `allow` buffer)
         bool has_ex; b2ip_exchange_t ex;
         cudaGraphExec_t exec;
         int coarse_launches, total_launches, slabs, sample_rows;
@@ -556,9 +559,10 @@ struct Guard {   // selects the index's device for the duration of a call
 
 // ------------------------------------------------------------------------- exact path
 // Scores qlist's queries (indices into q32) against the whole shard in fp32 and writes their
-// top-k.  qlist_dev == nullptr means queries [q_begin, q_begin + nql).
+// top-k.  qlist_dev == nullptr means queries [q_begin, q_begin + nql).  allow != nullptr
+// (filtered search): only rows whose bit is set may be returned.
 int exact_search(b2ip_handle h, const float* q32, const int* qlist_host, int64_t nql, int k,
-                 float* d_scores, int64_t* d_rows) {
+                 float* d_scores, int64_t* d_rows, const uint32_t* allow) {
     const int64_t n = h->n;
     RC_TRY(ensure(h, h->exact_scores, static_cast<size_t>(EXACT_QB) * n * sizeof(float)));
     const size_t misc_bytes = sizeof(ExactState) + EXACT_QB * 256 * sizeof(unsigned int) +
@@ -582,6 +586,11 @@ int exact_search(b2ip_handle h, const float* q32, const int* qlist_host, int64_t
         exact_scores_kernel<<<std::max(sgrid, 1), 256, sq_bytes, h->stream>>>(
             h->x32, h->x16, n, h->d, h->d_pad, h->sh, q32, qlist_dev + g0, nqg,
             reinterpret_cast<float*>(h->exact_scores.p));
+        if (allow) {
+            exact_mask_kernel<<<std::max(hgrid, 1), 256, 0, h->stream>>>(
+                reinterpret_cast<float*>(h->exact_scores.p), n, nqg, allow);
+            h->stats.total_launches++;
+        }
         exact_init_kernel<<<1, 256, 0, h->stream>>>(st, ghist, gcnt, k);
         for (int pass = 0; pass < 8; pass++) {
             exact_hist_kernel<<<dim3(std::max(hgrid, 1), nqg), 256, 0, h->stream>>>(
@@ -729,6 +738,9 @@ int tensor_search(b2ip_handle h, const float* q32, int64_t nq, int k, float* d_s
     const bool thr_round = h->ex && h->ex->gthr[0] && nq <= qb && h->ex->thr_stride >= nq && nq > 2048;
     h->ex_thr = thr_round;
     const bool fuse_refresh = h->fuse_refresh && !thr_round;
+    // filtered search: the coarse pass admits allowed rows only (DESIGN 4.1g)
+    const uint32_t* allow = h->filter;
+    const bool filtered = allow != nullptr;
     size_t ev_used = 0;
     std::vector<int> fallback;
 
@@ -754,7 +766,7 @@ int tensor_search(b2ip_handle h, const float* q32, int64_t nq, int k, float* d_s
         dyn = h->dyn_dev;
         for (auto& ge : h->graphs) {
             if (ge.nq == nq && ge.n == n && ge.k == k && ge.cap == cap && ge.ws_gen == h->ws_gen &&
-                ge.opt_gen == h->opt_gen && ge.has_ex == (h->ex != nullptr) &&
+                ge.opt_gen == h->opt_gen && ge.filtered == filtered && ge.has_ex == (h->ex != nullptr) &&
                 (!h->ex || memcmp(&ge.ex, h->ex, sizeof(b2ip_exchange_t)) == 0)) {
                 entry = &ge;
                 break;
@@ -807,7 +819,9 @@ int tensor_search(b2ip_handle h, const float* q32, int64_t nq, int k, float* d_s
         int64_t slab = std::min<int64_t>(cap, std::max<int64_t>(1024, 8ll * k));
         slab = slab / TILE_X * TILE_X;
         const int64_t first_slab = std::min<int64_t>(slab, n);
-        const bool dense_first = h->dense_first != 0;
+        // a filtered search runs its first slab through the counted filter at -inf instead: the
+        // positional store would list every row, disallowed ones included
+        const bool dense_first = h->dense_first != 0 && !filtered;
         CUtensorMap tmap_q;
         CAP_RC(make_tmap_bf16(h, &tmap_q, h->q16.p, pad_q(nqb), h->d_pad, TILE_Q));
         const bool use_pair = h->pair && nqb > TILE_Q && h->sm_count >= 2;
@@ -833,7 +847,8 @@ int tensor_search(b2ip_handle h, const float* q32, int64_t nq, int k, float* d_s
         // part of the corpus (k <= 42 at the default capacity).
         int boot_grid = 0;
         int64_t boot_tiles = 0;
-        if (use_stream && h->bootstrap && !h->dbg && n > slab)
+        // (not for a filtered search: the group maxima would include disallowed rows)
+        if (use_stream && h->bootstrap && !h->dbg && n > slab && !filtered)
             plan_bootstrap(n, k, cap, h->sm_count, h->d_pad, h->bootstrap_max_mb, &boot_grid, &boot_tiles);
         const bool bootstrap = boot_grid > 0;
         if (bootstrap) CAP_RC(ensure(h, h->gmax, static_cast<size_t>(nq_s) * boot_grid * STREAM_TILE_X * sizeof(uint32_t)));
@@ -922,7 +937,13 @@ int tensor_search(b2ip_handle h, const float* q32, int64_t nq, int k, float* d_s
             CAP_TRY(rec(e0));
             if (use_stream) {
                 const int grid = static_cast<int>(std::min<long long>(cp.x_tiles, h->sm_count));
-                if (nq_s == 32)
+                if (filtered && nq_s == 32)
+                    coarse_stream_kernel_bitmap<32><<<grid, COARSE_THREADS, stream_smem, h->stream>>>(
+                        tmap_q, tmap_x_pair, cp, stages, allow);
+                else if (filtered)
+                    coarse_stream_kernel_bitmap<64><<<grid, COARSE_THREADS, stream_smem, h->stream>>>(
+                        tmap_q, tmap_x_pair, cp, stages, allow);
+                else if (nq_s == 32)
                     coarse_stream_kernel<32><<<grid, COARSE_THREADS, stream_smem, h->stream>>>(
                         tmap_q, tmap_x_pair, cp, stages);
                 else
@@ -930,12 +951,20 @@ int tensor_search(b2ip_handle h, const float* q32, int64_t nq, int k, float* d_s
                         tmap_q, tmap_x_pair, cp, stages);
             } else if (use_pair) {
                 const int grid = 2 * static_cast<int>(std::min<long long>(tiles, h->sm_count / 2));
-                coarse_filter_pair_kernel<<<grid, COARSE_THREADS, PAIR_SMEM_BYTES, h->stream>>>(
-                    tmap_q, tmap_x_pair, cp);
+                if (filtered)
+                    coarse_filter_pair_kernel_bitmap<<<grid, COARSE_THREADS, PAIR_SMEM_BYTES, h->stream>>>(
+                        tmap_q, tmap_x_pair, cp, allow);
+                else
+                    coarse_filter_pair_kernel<<<grid, COARSE_THREADS, PAIR_SMEM_BYTES, h->stream>>>(
+                        tmap_q, tmap_x_pair, cp);
             } else {
                 const int grid = static_cast<int>(std::min<long long>(tiles, h->sm_count));
-                coarse_filter_kernel<false><<<grid, COARSE_THREADS, COARSE_SMEM_BYTES, h->stream>>>(
-                    tmap_q, tmap_x, cp);
+                if (filtered)
+                    coarse_filter_kernel_bitmap<<<grid, COARSE_THREADS, COARSE_SMEM_BYTES, h->stream>>>(
+                        tmap_q, tmap_x, cp, allow);
+                else
+                    coarse_filter_kernel<false><<<grid, COARSE_THREADS, COARSE_SMEM_BYTES, h->stream>>>(
+                        tmap_q, tmap_x, cp);
             }
             CAP_TRY(rec(e1));
             // the refresh after the LAST slab is fused into the finalize kernel -- unless this
@@ -1076,6 +1105,7 @@ int tensor_search(b2ip_handle h, const float* q32, int64_t nq, int k, float* d_s
             }
             b2ip_index_s::GraphEntry ge{};
             ge.nq = nq; ge.n = n; ge.k = k; ge.cap = cap; ge.ws_gen = h->ws_gen; ge.opt_gen = h->opt_gen;
+            ge.filtered = filtered;
             ge.has_ex = h->ex != nullptr;
             if (h->ex) ge.ex = *h->ex;
             ge.exec = exec;
@@ -1147,7 +1177,7 @@ int tensor_search(b2ip_handle h, const float* q32, int64_t nq, int k, float* d_s
     } else if (!fallback.empty()) {
         h->stats.fallback_queries = static_cast<int64_t>(fallback.size());
         RC_TRY(exact_search(h, q32, fallback.data(), static_cast<int64_t>(fallback.size()), k,
-                            d_scores, d_rows));
+                            d_scores, d_rows, allow));
         CU_TRY(h, cudaEventRecord(h->ev_t1, h->stream));
         CU_TRY(h, cudaStreamSynchronize(h->stream));
     }
@@ -1188,7 +1218,7 @@ int search_device(b2ip_handle h, int64_t nq, const float* dq, int k, float* d_sc
         h->stats.mode_used = B2IP_MODE_EXACT;
         std::vector<int> all(nq);
         for (int64_t i = 0; i < nq; i++) all[i] = static_cast<int>(i);
-        RC_TRY(exact_search(h, dq, all.data(), nq, k, d_scores, d_rows));
+        RC_TRY(exact_search(h, dq, all.data(), nq, k, d_scores, d_rows, h->filter));
     } else {
         h->stats.mode_used = B2IP_MODE_TENSOR;
         RC_TRY(tensor_search(h, dq, nq, k, d_scores, d_rows));   // records ev_t1 and synchronises
@@ -1650,6 +1680,11 @@ int b2ip_create_ex(int d, int device, int store_dtype, b2ip_handle* out) {
             cudaFuncSetAttribute(range_dense_kernel<ROWS_BF16, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, dense_smem) != cudaSuccess ||
             cudaFuncSetAttribute(range_dense_kernel<ROWS_F16, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, dense_smem) != cudaSuccess)
             return bail(B2IP_ERR_CUDA, "cudaFuncSetAttribute(MaxDynamicSharedMemorySize)");
+        if (cudaFuncSetAttribute(coarse_filter_kernel_bitmap, cudaFuncAttributeMaxDynamicSharedMemorySize, COARSE_SMEM_BYTES) != cudaSuccess ||
+            cudaFuncSetAttribute(coarse_filter_pair_kernel_bitmap, cudaFuncAttributeMaxDynamicSharedMemorySize, PAIR_SMEM_BYTES) != cudaSuccess ||
+            cudaFuncSetAttribute(coarse_stream_kernel_bitmap<32>, cudaFuncAttributeMaxDynamicSharedMemorySize, MAX_SMEM_OPTIN) != cudaSuccess ||
+            cudaFuncSetAttribute(coarse_stream_kernel_bitmap<64>, cudaFuncAttributeMaxDynamicSharedMemorySize, MAX_SMEM_OPTIN) != cudaSuccess)
+            return bail(B2IP_ERR_CUDA, "cudaFuncSetAttribute(MaxDynamicSharedMemorySize)");
     }
     h->gx = std::max(1, h->sm_count / 2);   // = clusters of the pair kernel: one query tile per wave,
                                             // the corpus tiles of a group stay L2 resident (measured best)
@@ -1673,7 +1708,7 @@ void b2ip_destroy(b2ip_handle h) {
     if (h->own_stream) cudaStreamSynchronize(h->own_stream);
     for (DevBuf* b : {&h->q16, &h->eps2, &h->thr, &h->cnt, &h->kept, &h->flags, &h->cand, &h->qstage, &h->qhalf,
                       &h->out_s, &h->out_r, &h->exact_scores, &h->exact_misc, &h->qlist, &h->stage,
-                      &h->seg_tab, &h->gmax})
+                      &h->seg_tab, &h->gmax, &h->allow})
         release(*b);
     range_release(h);
     if (h->v16.base || h->v32.base) {
@@ -1943,6 +1978,44 @@ int b2ip_search_ex(b2ip_handle h, int64_t nq, const void* queries_any, int q_dty
     RC_TRY(device_to_host(h, out_scores, h->out_s.p, sb));
     RC_TRY(device_to_host(h, out_rows, h->out_r.p, rb));
     return B2IP_OK;
+}
+
+int b2ip_search_filtered(b2ip_handle h, int64_t nq, const void* queries, int q_dtype, int k,
+                         const uint32_t* allow_bits, int64_t n_bits,
+                         float* out_scores, int64_t* out_rows, int mode, int mem) {
+    if (!h) return B2IP_ERR_INVALID;
+    if (n_bits != h->n)
+        return fail(h, B2IP_ERR_INVALID, "b2ip_search_filtered: n_bits=%lld, the index holds %lld rows",
+                    (long long)n_bits, (long long)h->n);
+    if (!allow_bits && n_bits > 0) return fail(h, B2IP_ERR_INVALID, "b2ip_search_filtered: NULL bitmap");
+    if (k < 1 || k > B2IP_MAX_K)
+        return fail(h, B2IP_ERR_INVALID, "b2ip_search_filtered: k=%d outside 1..%d", k, B2IP_MAX_K);
+    if (q_dtype != B2IP_F32 && q_dtype != B2IP_F16)
+        return fail(h, B2IP_ERR_INVALID, "b2ip_search_filtered: q_dtype=%d (use B2IP_F32 or B2IP_F16)", q_dtype);
+    if (mode < B2IP_MODE_AUTO || mode > B2IP_MODE_EXACT) return fail(h, B2IP_ERR_INVALID, "b2ip_search_filtered: mode=%d", mode);
+    if (mem != B2IP_MEM_HOST && mem != B2IP_MEM_DEVICE) return fail(h, B2IP_ERR_INVALID, "b2ip_search_filtered: mem=%d", mem);
+    Guard g(h->device);
+    // one copy per call into a library-owned buffer whose address stays put across calls (a
+    // captured small-batch graph reads it; the copy is queued ahead of the graph launch)
+    const size_t bytes = static_cast<size_t>((n_bits + 31) / 32) * sizeof(uint32_t);
+    if (bytes > 0 && mem == B2IP_MEM_DEVICE) {
+        // a device-to-device copy from a pageable host address is undefined: refuse it up front
+        cudaPointerAttributes a;
+        const bool on_device = cudaPointerGetAttributes(&a, allow_bits) == cudaSuccess &&
+                               (a.type == cudaMemoryTypeDevice || a.type == cudaMemoryTypeManaged);
+        cudaGetLastError();
+        if (!on_device)
+            return fail(h, B2IP_ERR_INVALID, "b2ip_search_filtered: mem=B2IP_MEM_DEVICE but allow_bits is not device memory");
+    }
+    if (bytes > 0) {
+        RC_TRY(ensure(h, h->allow, bytes));
+        CU_TRY(h, cudaMemcpyAsync(h->allow.p, allow_bits, bytes,
+                                  mem == B2IP_MEM_HOST ? cudaMemcpyHostToDevice : cudaMemcpyDeviceToDevice, h->stream));
+    }
+    h->filter = static_cast<const uint32_t*>(h->allow.p);
+    const int rc = b2ip_search_ex(h, nq, queries, q_dtype, k, out_scores, out_rows, mode, mem);
+    h->filter = nullptr;
+    return rc;
 }
 
 int b2ip_search_exchange(b2ip_handle h, int64_t nq, const float* queries_dev, int k,

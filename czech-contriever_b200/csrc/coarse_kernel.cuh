@@ -106,9 +106,13 @@ __device__ __forceinline__ void flush_hits(const CoarseParams& p, int q,
 // row's threshold.  Only if it passes (rare): branch-free hit mask, hits staged in shared
 // memory (flushed once per tile, after the accumulator is released) -- or, for dense chunks
 // (early slabs), appended straight from registers with one counter bump per chunk.
+// kFilter (filtered search): a hit is admitted only when its row's bit is set in `allow`.  Slabs
+// start at multiples of TILE_X (tensor_search), so the 32 rows of a chunk are exactly one word.
+template <bool kFilter = false>
 __device__ __forceinline__ void filter_accumulator(const CoarseParams& p, int q, float thr,
                                                    uint32_t taddr, long long x_row, int n_valid,
-                                                   unsigned long long* my_stage, int& n_staged) {
+                                                   unsigned long long* my_stage, int& n_staged,
+                                                   const uint32_t* allow = nullptr) {
 #pragma unroll 1
     for (int c = 0; c < TILE_X / 32; c++) {
         uint32_t v[32];
@@ -124,6 +128,9 @@ __device__ __forceinline__ void filter_accumulator(const CoarseParams& p, int q,
             const int vcols = n_valid - c * 32;          // columns of this chunk in range
             if (vcols < 32) mask &= vcols > 0 ? ((1u << vcols) - 1u) : 0u;
             const uint32_t row0 = static_cast<uint32_t>(x_row) + c * 32;
+            if constexpr (kFilter) {
+                if (mask) mask &= row_word(allow, row0);   // a set bit means row0 < x_row_end
+            }
             const int nh = __popc(mask);
             if (n_staged + nh > HIT_SLOTS) {
                 int slot = atomicAdd(p.cnt + q, nh);
@@ -178,10 +185,13 @@ __device__ __forceinline__ void dense_store_accumulator(const CoarseParams& p, i
     }
 }
 
-template <bool kDump>
-__global__ void __launch_bounds__(COARSE_THREADS, 1)
-coarse_filter_kernel(const __grid_constant__ CUtensorMap tmap_q,
-                     const __grid_constant__ CUtensorMap tmap_x, const CoarseParams p) {
+// The scoring kernels below are bodies shared by two entry points each: the search kernel and,
+// with kFilter, its filtered twin (`..._bitmap`), which takes the allowed-row bitmap as one more
+// kernel argument.  (A CoarseParams field would grow the struct and move the `stages` argument
+// of coarse_stream_kernel: the unfiltered kernels would no longer compile to the same code.)
+template <bool kDump, bool kFilter>
+__device__ __forceinline__ void coarse_filter_body(const CUtensorMap& tmap_q, const CUtensorMap& tmap_x,
+                                                   const CoarseParams p, const uint32_t* allow) {
     extern __shared__ uint8_t smem_raw[];
     // SWIZZLE_128B operand tiles need 1024-byte alignment.
     uint8_t* smem = reinterpret_cast<uint8_t*>(
@@ -319,7 +329,7 @@ coarse_filter_kernel(const __grid_constant__ CUtensorMap tmap_q,
             } else if (p.dense) {
                 dense_store_accumulator(p, q, taddr, x_row, n_valid);
             } else if (!(p.dbg & 4)) {
-                filter_accumulator(p, q, thr, taddr, x_row, n_valid, my_stage, n_staged);
+                filter_accumulator<kFilter>(p, q, thr, taddr, x_row, n_valid, my_stage, n_staged, allow);
             }
             // hand the accumulator back before touching global memory: the (latency-bound)
             // counter bump + key stores then overlap the MMAs of the following tiles
@@ -336,6 +346,20 @@ coarse_filter_kernel(const __grid_constant__ CUtensorMap tmap_q,
         ptx::tc_fence_after();
         ptx::tmem_dealloc<TMEM_COLS>(tmem_base);
     }
+}
+
+template <bool kDump>
+__global__ void __launch_bounds__(COARSE_THREADS, 1)
+coarse_filter_kernel(const __grid_constant__ CUtensorMap tmap_q,
+                     const __grid_constant__ CUtensorMap tmap_x, const CoarseParams p) {
+    coarse_filter_body<kDump, false>(tmap_q, tmap_x, p, nullptr);
+}
+
+__global__ void __launch_bounds__(COARSE_THREADS, 1)
+coarse_filter_kernel_bitmap(const __grid_constant__ CUtensorMap tmap_q,
+                            const __grid_constant__ CUtensorMap tmap_x, const CoarseParams p,
+                            const uint32_t* __restrict__ allow) {
+    coarse_filter_body<false, true>(tmap_q, tmap_x, p, allow);
 }
 
 // =======================================================================================
@@ -356,9 +380,9 @@ constexpr int PAIR_STAGE_BYTES = 2 * PAIR_HALF_BYTES;          // A half + B hal
 constexpr int PAIR_SMEM_BYTES =
     PAIR_STAGES * PAIR_STAGE_BYTES + 1024 + 256 + HIT_STAGE_BYTES;
 
-__global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(COARSE_THREADS, 1)
-coarse_filter_pair_kernel(const __grid_constant__ CUtensorMap tmap_q,
-                          const __grid_constant__ CUtensorMap tmap_x, const CoarseParams p) {
+template <bool kFilter>
+__device__ __forceinline__ void coarse_filter_pair_body(const CUtensorMap& tmap_q, const CUtensorMap& tmap_x,
+                                                        const CoarseParams p, const uint32_t* allow) {
     extern __shared__ uint8_t smem_raw[];
     uint8_t* smem = reinterpret_cast<uint8_t*>(
         (reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~static_cast<uintptr_t>(1023));
@@ -478,7 +502,8 @@ coarse_filter_pair_kernel(const __grid_constant__ CUtensorMap tmap_q,
             const uint32_t taddr =
                 tmem_base + (static_cast<uint32_t>(wq * 32) << 16) + static_cast<uint32_t>(as * TILE_X);
             if (p.dense) dense_store_accumulator(p, q, taddr, x_row, n_valid);
-            else if (!(p.dbg & 4)) filter_accumulator(p, q, thr, taddr, x_row, n_valid, my_stage, n_staged);
+            else if (!(p.dbg & 4))
+                filter_accumulator<kFilter>(p, q, thr, taddr, x_row, n_valid, my_stage, n_staged, allow);
             ptx::tc_fence_before();
             ptx::mbar_arrive_cluster(as == 0 ? tempty_leader0 : tempty_leader1);
             if (++as == 2) { as = 0; aphase ^= 1; }
@@ -494,6 +519,19 @@ coarse_filter_pair_kernel(const __grid_constant__ CUtensorMap tmap_q,
         ptx::tc_fence_after();
         ptx::tmem_dealloc_pair<TMEM_COLS>(tmem_base);
     }
+}
+
+__global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(COARSE_THREADS, 1)
+coarse_filter_pair_kernel(const __grid_constant__ CUtensorMap tmap_q,
+                          const __grid_constant__ CUtensorMap tmap_x, const CoarseParams p) {
+    coarse_filter_pair_body<false>(tmap_q, tmap_x, p, nullptr);
+}
+
+__global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(COARSE_THREADS, 1)
+coarse_filter_pair_kernel_bitmap(const __grid_constant__ CUtensorMap tmap_q,
+                                 const __grid_constant__ CUtensorMap tmap_x, const CoarseParams p,
+                                 const uint32_t* __restrict__ allow) {
+    coarse_filter_pair_body<true>(tmap_q, tmap_x, p, allow);
 }
 
 // =======================================================================================
@@ -526,12 +564,12 @@ constexpr int STREAM_MISC_BYTES = 1024 /*align*/ + 320 /*barriers*/;
 // disjoint, so the k-th largest group maximum is a lower bound of the k-th best score of the corpus:
 // bootstrap_threshold_kernel turns it into the admission threshold of the ONE filtered slab that
 // follows (instead of dense slab -> refresh -> small slab -> refresh -> main slab).
-template <int NQ, bool kGroupMax = false>
-__global__ void __launch_bounds__(COARSE_THREADS, 1)
-coarse_stream_kernel(const __grid_constant__ CUtensorMap tmap_q,
-                     const __grid_constant__ CUtensorMap tmap_x, const CoarseParams p,
-                     const int stages) {
+template <int NQ, bool kGroupMax, bool kFilter>
+__device__ __forceinline__ void coarse_stream_body(const CUtensorMap& tmap_q, const CUtensorMap& tmap_x,
+                                                   const CoarseParams p, const int stages,
+                                                   const uint32_t* allow) {
     static_assert(NQ == 32 || NQ == 64, "query batch is padded to 32 or 64 columns");
+    static_assert(!(kGroupMax && kFilter), "a filtered search takes no threshold bootstrap");
     constexpr uint32_t kTmemCols = STREAM_ACC * NQ;                  // 128 or 256: powers of two
     constexpr int Q_KB_BYTES = NQ * KBLOCK_BYTES;                     // one k-block of the batch
     extern __shared__ uint8_t smem_raw[];
@@ -668,7 +706,8 @@ coarse_stream_kernel(const __grid_constant__ CUtensorMap tmap_q,
             thr_r[j] = j < p.nq ? __ldg(p.thr + j) : __int_as_float(0x7f800000);   // +inf: padding
         for (int t = blockIdx.x; t < total_tiles; t += gridDim.x) {
             const long long row = p.x_row0 + static_cast<long long>(t) * STREAM_TILE_X + wq * 32 + lane;
-            const bool row_ok = row < p.x_row_end;
+            bool row_ok = row < p.x_row_end;
+            if constexpr (kFilter) row_ok = row_ok && row_allowed(allow, row);
             ptx::mbar_wait(&tfull_bar[as], aphase);
             ptx::tc_fence_after();
             const uint32_t taddr =
@@ -719,6 +758,22 @@ coarse_stream_kernel(const __grid_constant__ CUtensorMap tmap_q,
         ptx::tc_fence_after();
         ptx::tmem_dealloc<kTmemCols>(tmem_base);
     }
+}
+
+template <int NQ, bool kGroupMax = false>
+__global__ void __launch_bounds__(COARSE_THREADS, 1)
+coarse_stream_kernel(const __grid_constant__ CUtensorMap tmap_q,
+                     const __grid_constant__ CUtensorMap tmap_x, const CoarseParams p,
+                     const int stages) {
+    coarse_stream_body<NQ, kGroupMax, false>(tmap_q, tmap_x, p, stages, nullptr);
+}
+
+template <int NQ>
+__global__ void __launch_bounds__(COARSE_THREADS, 1)
+coarse_stream_kernel_bitmap(const __grid_constant__ CUtensorMap tmap_q,
+                            const __grid_constant__ CUtensorMap tmap_x, const CoarseParams p,
+                            const int stages, const uint32_t* __restrict__ allow) {
+    coarse_stream_body<NQ, false, true>(tmap_q, tmap_x, p, stages, allow);
 }
 
 }  // namespace b2ip

@@ -38,4 +38,13 @@ __host__ __device__ __forceinline__ float key_score(unsigned long long k) {
     return unorder_f32(static_cast<uint32_t>(k >> 32));
 }
 
+// Allowed-row bitmap of a filtered search (b2ip_search_filtered): bit r & 31 of word r >> 5 is
+// set when local row r may be returned.
+__device__ __forceinline__ uint32_t row_word(const uint32_t* allow, uint32_t row) {
+    return __ldg(allow + (row >> 5));
+}
+__device__ __forceinline__ bool row_allowed(const uint32_t* allow, long long row) {
+    return (__ldg(allow + (row >> 5)) >> (row & 31)) & 1u;
+}
+
 }  // namespace b2ip

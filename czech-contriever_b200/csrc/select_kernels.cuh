@@ -1267,6 +1267,18 @@ exact_scores_kernel(const float* __restrict__ x32, const __nv_bfloat16* __restri
     }
 }
 
+// Filtered search: every row the bitmap does not allow gets a NaN score, which the select below
+// never reports (order(NaN) = 0), so the group's answer is that of the allowed rows alone.
+__global__ void __launch_bounds__(256)
+exact_mask_kernel(float* __restrict__ scores /*[EXACT_QB, n]*/, long long n, int nqg,
+                  const uint32_t* __restrict__ allow) {
+    for (long long r = static_cast<long long>(blockIdx.x) * blockDim.x + threadIdx.x; r < n;
+         r += static_cast<long long>(gridDim.x) * blockDim.x) {
+        if (!row_allowed(allow, r))
+            for (int b = 0; b < nqg; b++) scores[static_cast<long long>(b) * n + r] = __int_as_float(0x7fc00000);
+    }
+}
+
 // per-query select state of the exact path
 struct ExactState {
     unsigned long long prefix[EXACT_QB];

@@ -157,6 +157,19 @@ int b2ip_search(b2ip_handle h, int64_t nq, const float* queries, int k, float* o
 int b2ip_search_ex(b2ip_handle h, int64_t nq, const void* queries, int q_dtype, int k,
                    float* out_scores, int64_t* out_rows, int mode, int mem);
 
+/* index.search(q, k, params=SearchParameters(sel=IDSelectorBitmap)): b2ip_search_ex restricted to the
+ * local rows whose bit is set in allow_bits (bit r&31 of word r>>5, n_bits == ntotal; NULL allowed
+ * only when n_bits == 0).  allow_bits lives where `mem` says, like the queries.  Bits past n_bits
+ * in the last word are ignored.  The answer is exactly b2ip_search_ex's on an index holding only
+ * the allowed rows in their original order, ids mapped back to the original rows (row offset or
+ * segments as usual): same tie rule, NaN rows never returned, (-FLT_MAX, -1) padding when fewer
+ * than k allowed rows have a non-NaN score, bit-identical scores.  One bitmap per call, shared by
+ * all queries.  A bad n_bits, NULL bitmap, mode, k or q_dtype, or mem = B2IP_MEM_DEVICE with a
+ * bitmap that is not device memory, gives B2IP_ERR_INVALID. */
+int b2ip_search_filtered(b2ip_handle h, int64_t nq, const void* queries, int q_dtype, int k,
+                         const uint32_t* allow_bits, int64_t n_bits,
+                         float* out_scores, int64_t* out_rows, int mode, int mem);
+
 /* replaces lims, D, I = index.range_search(q, radius) (faiss IndexFlatIP).
  * queries [nq,d] fp32 or fp16 (q_dtype), mode B2IP_MODE_AUTO/TENSOR/EXACT.  Computes the answer,
  * keeps it in library memory and writes the host array out_lims[nq+1] (out_lims[nq] = total).
